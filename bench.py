@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this framework (CUDA, libcassie2d.so)
   python bench.py --impl reference --gpus N ...            # the CPU restatement on the host cores
+  python bench.py ... --dump-outputs DIR                   # + the last timed step's results as DIR/<name>.npy
 
 A "step" is one launch of the fused step kernel: `--substeps` (default 10, the Python envs' n,
 cassie2d.py:97) simulator steps of dt = 0.5 ms for every env of the batch, with the controller of
@@ -68,6 +69,9 @@ def parse():
     p.add_argument("--ref-envs", type=int, default=1024, help="--impl reference: envs of the bounded CPU sample")
     p.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                    help="weak: --envs per GPU (the driver's contract); strong: --envs in TOTAL, split evenly over the ranks")
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write what the last timed step returned to its caller as DIR/<name>.npy "
+                        "(rank r of several writes DIR/<name>_rank<r>.npy), for output-for-output comparison of two builds")
     return p.parse_args()
 
 
@@ -281,6 +285,27 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm), "source": "nvidia-smi -lms 100"}
 
 
+# ----------------------------------------------------------------------------- output dump
+DUMP_BYTES = 60 * 10**6   # keeps a dump, .npy headers included, under 64 MB
+
+
+def dump_outputs(d, arrays, suffix=""):
+    """Writes `arrays` (name -> tensor with one row per env) as d/<name><suffix>.npy in float32, or float64 where the
+    path computed in fp64.  Above DUMP_BYTES in all, the same seeded sample of envs is taken from every array and
+    env_index<suffix>.npy lists the env indices of its rows."""
+    host = {k: v.cpu().numpy() for k, v in arrays.items()}
+    host = {k: a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False) for k, a in host.items()}
+    n = len(next(iter(host.values())))
+    row_bytes = sum(a.nbytes for a in host.values()) // n
+    if n * row_bytes > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // (row_bytes + 8), replace=False))
+        host = {k: a[keep] for k, a in host.items()}
+        host["env_index"] = keep.astype(np.float64)
+    os.makedirs(d, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(d, k + suffix + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- native arm
 def run_native(args):
     import torch
@@ -338,7 +363,7 @@ def run_native(args):
         elif wl == "torque_random":
             b.step_torque(acts[k], sub)
         else:
-            obj.step(acts[k], n=sub)
+            return obj.step(acts[k], n=sub)
 
     def barrier():
         if world > 1:
@@ -371,7 +396,7 @@ def run_native(args):
     for k in range(args.steps):
         flush.zero_()                                   # L2 flush, outside the timed events
         ev[k][0].record()
-        one_step(n_pre + args.warmup + k)
+        last = one_step(n_pre + args.warmup + k)
         ev[k][1].record()
     barrier()
     launches = L.CassieKernelLaunchCount() - launches0
@@ -383,6 +408,11 @@ def run_native(args):
     ms_max = float(t.item())
     # rollout statistics (NCCL reduce, outside the timed region): mean pelvis height, envs below 0.5 m
     s = b.get_general_state()
+    if args.dump_outputs:
+        out = {"general_state": s, "operational_space_state": b.get_operational_space_state()}
+        if wl == "pd_env":
+            out.update(zip(("obs", "reward", "done"), last))
+        dump_outputs(args.dump_outputs, out, "_rank%d" % rank if world > 1 else "")
     stats = torch.stack([s[:, 1].double().sum(), (s[:, 1] < 0.5).double().sum(), (~torch.isfinite(s).all(dim=1)).double().sum()])
     if world > 1:
         dist.all_reduce(stats)

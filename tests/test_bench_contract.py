@@ -43,6 +43,28 @@ def test_native_arm_refuses_cpu():
     assert r.returncode != 0 and "no CUDA device" in (r.stderr + r.stdout)
 
 
+@pytest.mark.gpu
+@pytest.mark.parametrize("workload", ["squat_osc", "pd_env"])
+def test_dump_outputs_repeat_bit_for_bit(workload, tmp_path):
+    """--dump-outputs writes the last timed step's results; the same arguments give the same inputs, hence the same files"""
+    import numpy as np
+    n = 512
+    names = ("obs", "reward", "done") if workload == "pd_env" else ()
+    dumps = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        r = _run(["--workload", workload, "--envs", str(n), "--steps", "3", "--warmup", "1", "--preadvance", "20",
+                  "--no-cpu-baseline", "--dump-outputs", str(d)])
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])["steps"] == 3
+        dumps.append({f.stem: np.load(f) for f in sorted(d.glob("*.npy"))})
+    shapes = {"general_state": (n, 26), "operational_space_state": (n, 18), "obs": (n, 17), "reward": (n,), "done": (n,)}
+    assert sorted(dumps[0]) == sorted(("general_state", "operational_space_state") + names)
+    for name, a in dumps[0].items():
+        assert a.shape == shapes[name] and a.dtype == np.float32 and np.isfinite(a).all()
+        assert np.array_equal(a, dumps[1][name]), name
+
+
 def test_traffic_stamp_matches_sources():
     """profiles/traffic.json carries the hash of the kernel sources its ncu capture ran; bench.py prints the number only
     while they are the sources being timed"""
