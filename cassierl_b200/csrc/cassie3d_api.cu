@@ -52,6 +52,10 @@ struct Cassie3dBatch {
   void* d_reset_qd = nullptr;
   void* d_action = nullptr;   // host-variant staging
   uint8_t* d_done = nullptr;
+  void* d_obs = nullptr;      // host-variant staging of EnvStepHost
+  void* d_reward = nullptr;
+  int32_t* ep_len = nullptr;  // [n] policy steps since the env's last reset (EnvStep)
+  std::vector<double> kp, kd; // PD gains of the env's kActPd action space, per motor
   cudaStream_t own_stream = nullptr;
   size_t rs() const { return precision == 64 ? 8 : 4; }
 };
@@ -83,7 +87,8 @@ int setup(Cassie3dBatch* h, TreeBatchView<T>& v) {
       dmalloc(h, (void**)&v.order, sizeof(int32_t) * n) || dmalloc(h, (void**)&v.bins, sizeof(int32_t) * 2 * kTreeBins) ||
       dmalloc(h, (void**)&v.resume, sizeof(int32_t) * n) || dmalloc(h, &h->d_reset_q, sizeof(T) * m.nq) ||
       dmalloc(h, &h->d_reset_qd, sizeof(T) * m.nv) || dmalloc(h, &h->d_action, sizeof(T) * n * m.nu) ||
-      dmalloc(h, (void**)&h->d_done, n))
+      dmalloc(h, (void**)&h->d_done, n) || dmalloc(h, &h->d_obs, sizeof(T) * n * kObsDim3d) ||
+      dmalloc(h, &h->d_reward, sizeof(T) * n) || dmalloc(h, (void**)&h->ep_len, sizeof(int32_t) * n))
     return -1;
   return 0;
 }
@@ -111,7 +116,43 @@ int step(Cassie3dBatch* h, const void* action, int n_sub, double z_done, int aut
   CU3_OK(TreeLaunch<T>::step(model_of<T>(h), view<T>(h), a, h->lanes, s));
   return 0;
 }
+
+template <typename T>
+int env_step(Cassie3dBatch* h, int mode, const void* action, int n_sub, int max_path_length, int flags, void* obs, void* reward,
+             uint8_t* done, cudaStream_t s) {
+  TreeStepArgs a;
+  a.action = action; a.n_sub = n_sub; a.z_done = 0; a.auto_reset = 0; a.done = done;
+  a.reset_q = h->d_reset_q; a.reset_qd = h->d_reset_qd;
+  TreeEnvParams<T> ep;
+  for (int i = 0; i < kMaxAct; i++) {
+    ep.kp[i] = i < h->model.nu ? (T)h->kp[i] : (T)0;
+    ep.kd[i] = i < h->model.nu ? (T)h->kd[i] : (T)0;
+  }
+  ep.mode = mode; ep.flags = flags; ep.max_path_length = max_path_length;
+  ep.obs = (T*)obs; ep.reward = (T*)reward; ep.ep_len = h->ep_len;
+  CU3_OK(TreeLaunch<T>::env_step(model_of<T>(h), view<T>(h), a, ep, h->lanes, s));
+  return 0;
+}
+
+template <typename T>
+int observe(Cassie3dBatch* h, void* obs, cudaStream_t s) {
+  CU3_OK(TreeLaunch<T>::observe(model_of<T>(h), view<T>(h), (T*)obs, s));
+  return 0;
+}
+
+int check_env_step(Cassie3dBatch* h, int mode, const void* action, int n_substeps, int flags) {
+  if (!h) return fail3("null handle");
+  if (mode != CASSIE3D_MODE_TORQUE && mode != CASSIE3D_MODE_PD) return fail3("mode must be CASSIE3D_MODE_TORQUE or CASSIE3D_MODE_PD");
+  if (!action) return fail3("EnvStep needs an action");
+  if (n_substeps < 1) return fail3("n_substeps must be at least 1");
+  if (flags & ~(CASSIE3D_AUTO_RESET | CASSIE3D_TERMINAL_OBS)) return fail3("unknown flag bits");
+  return 0;
+}
 }  // namespace
+
+static_assert((int)CASSIE3D_MODE_TORQUE == (int)kActTorque && (int)CASSIE3D_MODE_PD == (int)kActPd, "action modes");
+static_assert((int)CASSIE3D_AUTO_RESET == (int)kEnvAutoReset && (int)CASSIE3D_TERMINAL_OBS == (int)kEnvTerminalObs, "env flags");
+static_assert((int)CASSIE3D_OBS_DIM == kObsDim3d, "observation size");
 
 #define DISPATCH3(h, expr32, expr64) ((h)->precision == 64 ? (expr64) : (expr32))
 
@@ -150,6 +191,8 @@ Cassie3dBatch* Cassie3dBatchCreate(const char* xml_path, int n_envs, int device,
     for (int i = 0; i < 7; i++) { h->reset_q[7 + i] = leg[i]; h->reset_q[14 + i] = leg[i]; }
   }
   if (DISPATCH3(h, upload_reset<float>(h), upload_reset<double>(h))) { Cassie3dBatchDestroy(h); return nullptr; }
+  h->kp.assign(m.nu, kDefaultKp);
+  h->kd.assign(m.nu, kDefaultKd);
   if (cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking) != cudaSuccess) { fail3("cudaStreamCreate"); Cassie3dBatchDestroy(h); return nullptr; }
   if (Cassie3dBatchResetAll(h, nullptr, nullptr)) { Cassie3dBatchDestroy(h); return nullptr; }
   cudaDeviceSynchronize();
@@ -203,6 +246,12 @@ int Cassie3dBatchResetAll(Cassie3dBatch* h, const uint8_t* mask, void* stream) {
     CU3_OK(TreeLaunch<double>::set_all(h->v64, h->model.nq, h->model.nv, (const double*)h->d_reset_q, (const double*)h->d_reset_qd, mask, s));
   else
     CU3_OK(TreeLaunch<float>::set_all(h->v32, h->model.nq, h->model.nv, (const float*)h->d_reset_q, (const float*)h->d_reset_qd, mask, s));
+  if (mask) {
+    k_tree_zero_len<<<(h->n + 127) / 128, 128, 0, s>>>(h->n, mask, h->ep_len);
+    count_launch();
+    CU3_OK(cudaGetLastError());
+  } else
+    CU3_OK(cudaMemsetAsync(h->ep_len, 0, sizeof(int32_t) * (size_t)h->n, s));
   return 0;
 }
 
@@ -220,6 +269,7 @@ int Cassie3dBatchSetState(Cassie3dBatch* h, const void* qpos, const void* qvel, 
   CU3_OK(cudaMemcpyAsync(qpos_of(h), qpos, h->rs() * n * h->model.nq, cudaMemcpyDeviceToDevice, s));
   CU3_OK(cudaMemcpyAsync(qvel_of(h), qvel, h->rs() * n * h->model.nv, cudaMemcpyDeviceToDevice, s));
   CU3_OK(cudaMemsetAsync(warm_of(h), 0, h->rs() * n * h->model.nv, s));
+  CU3_OK(cudaMemsetAsync(h->ep_len, 0, sizeof(int32_t) * n, s));
   return 0;
 }
 
@@ -285,6 +335,59 @@ int Cassie3dBatchGetResets(Cassie3dBatch* h, int32_t* resets, void* stream) {
   if (!h || !resets) return fail3("null argument");
   DeviceGuard g(h->device);
   CU3_OK(cudaMemcpyAsync(resets, resets_of(h), sizeof(int32_t) * (size_t)h->n, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return 0;
+}
+
+int Cassie3dBatchSetPdGains(Cassie3dBatch* h, const double* kp, const double* kd) {
+  if (!h || !kp || !kd) return fail3("null argument");
+  h->kp.assign(kp, kp + h->model.nu);
+  h->kd.assign(kd, kd + h->model.nu);
+  return 0;
+}
+
+int Cassie3dBatchEnvStep(Cassie3dBatch* h, int mode, const void* action, int n_substeps, int max_path_length, int flags,
+                         void* obs, void* reward, uint8_t* done, void* stream) {
+  if (check_env_step(h, mode, action, n_substeps, flags)) return -1;
+  if (!obs || !reward || !done) return fail3("null argument");
+  DeviceGuard g(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  return DISPATCH3(h, env_step<float>(h, mode, action, n_substeps, max_path_length, flags, obs, reward, done, s),
+                   env_step<double>(h, mode, action, n_substeps, max_path_length, flags, obs, reward, done, s));
+}
+
+int Cassie3dBatchEnvStepHost(Cassie3dBatch* h, int mode, const void* action, int n_substeps, int max_path_length, int flags,
+                             void* obs_out, void* reward_out, uint8_t* done_out) {
+  if (check_env_step(h, mode, action, n_substeps, flags)) return -1;
+  DeviceGuard g(h->device);
+  cudaStream_t s = h->own_stream;
+  const size_t n = (size_t)h->n;
+  CU3_OK(cudaMemcpyAsync(h->d_action, action, h->rs() * n * h->model.nu, cudaMemcpyHostToDevice, s));
+  if (DISPATCH3(h, env_step<float>(h, mode, h->d_action, n_substeps, max_path_length, flags, h->d_obs, h->d_reward, h->d_done, s),
+                env_step<double>(h, mode, h->d_action, n_substeps, max_path_length, flags, h->d_obs, h->d_reward, h->d_done, s)))
+    return -1;
+  if (obs_out) CU3_OK(cudaMemcpyAsync(obs_out, h->d_obs, h->rs() * n * kObsDim3d, cudaMemcpyDeviceToHost, s));
+  if (reward_out) CU3_OK(cudaMemcpyAsync(reward_out, h->d_reward, h->rs() * n, cudaMemcpyDeviceToHost, s));
+  if (done_out) CU3_OK(cudaMemcpyAsync(done_out, h->d_done, n, cudaMemcpyDeviceToHost, s));
+  CU3_OK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+int Cassie3dBatchEnvReset(Cassie3dBatch* h, const uint8_t* mask, void* obs, void* stream) {
+  if (Cassie3dBatchResetAll(h, mask, stream)) return -1;
+  return obs ? Cassie3dBatchObserve(h, obs, stream) : 0;
+}
+
+int Cassie3dBatchObserve(Cassie3dBatch* h, void* obs, void* stream) {
+  if (!h || !obs) return fail3("null argument");
+  DeviceGuard g(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  return DISPATCH3(h, observe<float>(h, obs, s), observe<double>(h, obs, s));
+}
+
+int Cassie3dBatchGetEpisodeLengths(Cassie3dBatch* h, int32_t* ep_len, void* stream) {
+  if (!h || !ep_len) return fail3("null argument");
+  DeviceGuard g(h->device);
+  CU3_OK(cudaMemcpyAsync(ep_len, h->ep_len, sizeof(int32_t) * (size_t)h->n, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return 0;
 }
 

@@ -967,6 +967,24 @@ bool flatten_tree(const Model3& M, tree::TreeModel<double>* out, std::string* er
     if (d < 0) { *err = "motor on unknown joint '" + mo.joint + "'"; return false; }
     m.act_dof[a] = d; m.act_gear[a] = mo.gear; m.act_limited[a] = mo.limited ? 1 : 0; m.act_lo[a] = mo.lo; m.act_hi[a] = mo.hi;
   }
+  // ---- foot sites of the env observation (a foot = the mean of its front and rear contact site), in the link frame
+  static const char* const foot_sites[kNumFootSites] = {"left_contact_front", "left_contact_rear", "right_contact_front", "right_contact_rear"};
+  for (int k = 0; k < kNumFootSites; k++) {
+    int found = 0;
+    for (int b = 1; b < nb; b++)
+      for (auto& s : M.bodies[b].sites)
+        if (s.name == foot_sites[k]) {
+          const V3 p = in_link[b].p + mul(in_link[b].R, s.pos);
+          m.site_link[k] = link_of[b];
+          m.site_pos[k][0] = p.x; m.site_pos[k][1] = p.y; m.site_pos[k][2] = p.z;
+          found++;
+        }
+    if (found != 1) {
+      *err = std::string(found ? "more than one site named '" : "the model has no site named '") + foot_sites[k] +
+             "' (the 3-D env observes the feet at the sites left/right_contact_front/rear)";
+      return false;
+    }
+  }
   return true;
 }
 

@@ -192,6 +192,42 @@ template <typename T> TREE_HD void jac_col(T* r, const T* S, const T* P) {
 }
 
 // ---------------------------------------------------------------------------------------------- kinematics + dynamics
+// One link's frame (orientation, position about the base position): the frame part of link_pass below, the same
+// arithmetic, for the env's frame pass (tree_env.cuh).  A hinge link also returns its joint's anchor `an` and axis `ax`
+// in world axes.  Needs the parent's frame.
+template <typename T, typename SC>
+TREE_FN void link_frame(const TreeModel<T>& m, SC& s, int l, T* an, T* ax) {
+  T* pos = s.xpos[l];
+  T* mat = s.xmat[l];
+  if (l == 0) {
+    T w = s.q[3], x = s.q[4], y = s.q[5], z = s.q[6];
+    const T nq = (T)1 / sqrt(w * w + x * x + y * y + z * z);   // mj_normalizeQuat
+    w *= nq; x *= nq; y *= nq; z *= nq;
+    mat[0] = 1 - 2 * (y * y + z * z); mat[1] = 2 * (x * y - w * z); mat[2] = 2 * (x * z + w * y);
+    mat[3] = 2 * (x * y + w * z); mat[4] = 1 - 2 * (x * x + z * z); mat[5] = 2 * (y * z - w * x);
+    mat[6] = 2 * (x * z - w * y); mat[7] = 2 * (y * z + w * x); mat[8] = 1 - 2 * (x * x + y * y);
+    pos[0] = pos[1] = pos[2] = 0;
+  } else {
+    const int p = m.parent[l];
+    T R0[9], t[3];
+    mulm(R0, s.xmat[p], m.lmat[l]);
+    mulv(t, s.xmat[p], m.lpos[l]);
+    mulv(an, R0, m.jpos[l]);
+    for (int i = 0; i < 3; i++) an[i] += s.xpos[p][i] + t[i];
+    mulv(ax, R0, m.axis[l]);
+    // rotation about the hinge axis, in the link frame (Rodrigues)
+    const T th = s.q[6 + l] - m.ref[l];
+    const T sn = sin(th), cs = cos(th), vc = 1 - cs;
+    const T* a = m.axis[l];
+    T Rl[9] = {cs + a[0] * a[0] * vc, a[0] * a[1] * vc - a[2] * sn, a[0] * a[2] * vc + a[1] * sn,
+               a[1] * a[0] * vc + a[2] * sn, cs + a[1] * a[1] * vc, a[1] * a[2] * vc - a[0] * sn,
+               a[2] * a[0] * vc - a[1] * sn, a[2] * a[1] * vc + a[0] * sn, cs + a[2] * a[2] * vc};
+    mulm(mat, R0, Rl);
+    mulv(t, mat, m.jpos[l]);
+    for (int i = 0; i < 3; i++) pos[i] = an[i] - t[i];
+  }
+}
+
 // One link: frame, motion subspace, velocity, velocity-product acceleration, own spatial inertia and RNE force.
 template <typename T, typename SC>
 TREE_FN void link_pass(const TreeModel<T>& m, SC& s, int l) {

@@ -7,6 +7,7 @@
 #include <cstdlib>
 #include <cuda_runtime.h>
 #include "tree_engine.cuh"
+#include "tree_env.cuh"
 
 namespace cassie {
 void count_launch();
@@ -118,6 +119,96 @@ k_tree_step(const __grid_constant__ TreeModel<T> m, const TreeBatchView<T> v, co
   }
 }
 
+// What the env variant of the step kernel (k_tree_env_step, Cassie3dBatchEnvStep) adds: the action space, the
+// stand task's epilogue (tree_env.cuh) and its outputs.  A __grid_constant__ parameter: the gains are read from the
+// constant bank with tile-uniform addresses.
+template <typename T>
+struct TreeEnvParams {
+  T kp[kMaxAct], kd[kMaxAct];   // PD gains of the handle
+  int mode;                     // kActTorque: the action is the controls; kActPd: PD targets, the law runs every substep
+  int flags;                    // kEnvAutoReset, kEnvTerminalObs
+  int max_path_length;          // > 0: done = 3 when the episode length reaches it
+  T* obs;                       // [n][kObsDim3d]
+  T* reward;                    // [n]
+  int32_t* ep_len;              // [n] policy steps since the env's last reset
+};
+
+// the env kernels' per-env scratch: the step's, plus the action as given (PD targets survive all substeps in it)
+template <typename T, int ROWS, int CON>
+struct EnvScratch : Scratch<T, ROWS, CON> {
+  T target[kMaxAct];
+};
+
+// Cassie3dBatchEnvStep: the passes of k_tree_step (same MODEs, same physics) with the env's action space -- in kActPd the
+// PD law runs ahead of every substep on the targets kept in s.target, which the continuation pass re-reads from `action`
+// -- and, instead of the z_done rule, the stand task's epilogue (tree_env.cuh).  The epilogue runs in the pass that
+// completes the env's last substep, so exactly once per env and call.  A separate kernel, so that k_tree_step is
+// compiled exactly as without the env.
+template <typename T, int LANES, int ROWS, int CON, int MODE>
+__global__ void __launch_bounds__(kTreeMaxBlock)
+k_tree_env_step(const __grid_constant__ TreeModel<T> m, const TreeBatchView<T> v, const __grid_constant__ TreeEnvParams<T> env,
+                const T* __restrict__ action, int n_sub, uint8_t* __restrict__ done, const T* __restrict__ reset_q,
+                const T* __restrict__ reset_qd, int step_barrier) {
+  typedef EnvScratch<T, ROWS, CON> SC;
+  extern __shared__ __align__(16) unsigned char tree_smem[];
+  const Tile<LANES> tl = Tile<LANES>::make();
+  const int tile_in_block = (int)threadIdx.x / LANES, tiles_per_block = (int)blockDim.x / LANES;
+  const int e_raw = (int)blockIdx.x * tiles_per_block + tile_in_block;
+  const bool active = e_raw < v.n;
+  const int e = active ? e_raw : v.n - 1;
+  int k0 = 0;
+  if (MODE == 2) {
+    k0 = v.resume[e];
+    if (!active || k0 >= n_sub) return;
+  }
+  SC& s = *reinterpret_cast<SC*>(tree_smem + (size_t)tile_in_block * sizeof(SC));
+  const int nq = m.nq, nv = m.nv, nu = m.nu;
+  const T* gq = v.qpos + (size_t)e * nq;
+  const T* gv = v.qvel + (size_t)e * nv;
+  const T* gw = v.warm + (size_t)e * nv;
+  for (int i = tl.lane; i < 7; i += LANES) s.q[i] = gq[i];
+  for (int d = 6 + tl.lane; d < nv; d += LANES) s.q[d + 1] = gq[m.user_dof[d] + 1];
+  for (int d = tl.lane; d < nv; d += LANES) { s.qd[d] = gv[m.user_dof[d]]; s.warm[d] = gw[m.user_dof[d]]; }
+  for (int a = tl.lane; a < nu; a += LANES) s.target[a] = s.ctrl[a] = action[(size_t)e * nu + a];
+  if (tl.lane == 0) { s.n_dropped = 0; s.overflow = 0; }
+  tl.sync();
+  TreeStats st = {0, 0, 0, 0};
+  int k_done = n_sub;
+  bool alive = true;
+  const bool pd = env.mode == kActPd;
+  for (int k = k0; k < n_sub; k++) {
+    if (MODE != 2 && step_barrier > 0 && k % step_barrier == 0) __syncthreads();
+    if (!alive) continue;
+    if (pd) pd_controls(tl, m, s, s.target, env.kp, env.kd);
+    if (!tree_step(tl, m, s, s.ctrl, &st, MODE == 1)) { alive = false; k_done = k; }
+  }
+  if (!active) return;                       // no CTA barrier follows
+  EnvResult r = {0, 0, false};
+  if (alive) {                               // not for an env that is handed on
+    T rew;
+    r = env_finish(tl, m, s, s.target, env.flags, env.max_path_length, reset_q, reset_qd, env.ep_len[e],
+                   env.obs + (size_t)e * kObsDim3d, &rew);
+    if (tl.lane == 0) { env.reward[e] = rew; env.ep_len[e] = r.len; }
+  }
+  T* oq = v.qpos + (size_t)e * nq;
+  T* ov = v.qvel + (size_t)e * nv;
+  T* ow = v.warm + (size_t)e * nv;
+  for (int i = tl.lane; i < 7; i += LANES) oq[i] = s.q[i];
+  for (int d = 6 + tl.lane; d < nv; d += LANES) oq[m.user_dof[d] + 1] = s.q[d + 1];
+  for (int d = tl.lane; d < nv; d += LANES) { ov[m.user_dof[d]] = s.qd[d]; ow[m.user_dof[d]] = s.warm[d]; }
+  if (tl.lane == 0) {
+    if (MODE != 0) v.resume[e] = k_done;
+    if (alive) {
+      done[e] = (uint8_t)r.done;
+      if (n_sub > k0) {
+        v.stats[4 * e + 0] = st.nefc; v.stats[4 * e + 1] = st.ncon; v.stats[4 * e + 2] = st.sweeps;
+        v.stats[4 * e + 3] += st.dropped;
+      }
+      if (r.reset) v.resets[e] += 1;
+    }
+  }
+}
+
 // ---- binning of the envs by the constraint-row count of their last step (a counting sort in three tiny launches)
 static __global__ void k_tree_bin_hist(int n, const int32_t* __restrict__ stats, int32_t* __restrict__ bins) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -148,10 +239,47 @@ __global__ void k_tree_set_all(TreeBatchView<T> v, int nq, int nv, const T* __re
   for (int i = 0; i < nv; i++) { v.qvel[(size_t)e * nv + i] = qd[i]; v.warm[(size_t)e * nv + i] = 0; }
 }
 
+// the env observation of every env's current state, without stepping (Cassie3dBatchObserve / EnvReset): a tile of
+// kObsLanes lanes per env, the frame pass on a small shared block (state and frames only)
+template <typename T>
+struct FrameScratch {
+  T q[kMaxDof + 1], qd[kMaxDof];
+  T xpos[kMaxLinks][3], xmat[kMaxLinks][9];
+};
+constexpr int kObsLanes = 8, kObsTiles = 16;
+
+template <typename T>
+__global__ void __launch_bounds__(kObsLanes * kObsTiles)
+k_tree_observe(const __grid_constant__ TreeModel<T> m, const TreeBatchView<T> v, T* __restrict__ obs) {
+  __shared__ FrameScratch<T> sm[kObsTiles];
+  const Tile<kObsLanes> tl = Tile<kObsLanes>::make();
+  const int t = (int)threadIdx.x / kObsLanes, e = (int)blockIdx.x * kObsTiles + t;
+  if (e >= v.n) return;                      // whole tiles leave: only tile barriers follow
+  FrameScratch<T>& s = sm[t];
+  const T* gq = v.qpos + (size_t)e * m.nq;
+  const T* gv = v.qvel + (size_t)e * m.nv;
+  for (int i = tl.lane; i < 7; i += kObsLanes) s.q[i] = gq[i];
+  for (int d = 6 + tl.lane; d < m.nv; d += kObsLanes) s.q[d + 1] = gq[m.user_dof[d] + 1];
+  for (int d = tl.lane; d < m.nv; d += kObsLanes) s.qd[d] = gv[m.user_dof[d]];
+  tl.sync();
+  T f[6];
+  observe(tl, m, s, obs + (size_t)e * kObsDim3d, f);
+}
+
+// episode lengths of the selected envs (mask nullptr: all) <- 0
+static __global__ void k_tree_zero_len(int n, const uint8_t* __restrict__ mask, int32_t* __restrict__ ep_len) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < n && (!mask || mask[e])) ep_len[e] = 0;
+}
+
 template <typename T>
 struct TreeLaunch {
   static cudaError_t step(const TreeModel<T>& m, const TreeBatchView<T>& v, const TreeStepArgs& a, int lanes, cudaStream_t s);
   static cudaError_t set_all(const TreeBatchView<T>& v, int nq, int nv, const T* q, const T* qd, const uint8_t* mask, cudaStream_t s);
+  // EnvStep: a.action (required), a.n_sub, a.done, a.reset_q / reset_qd are used; z_done / auto_reset are the env's rule
+  static cudaError_t env_step(const TreeModel<T>& m, const TreeBatchView<T>& v, const TreeStepArgs& a, const TreeEnvParams<T>& env,
+                              int lanes, cudaStream_t s);
+  static cudaError_t observe(const TreeModel<T>& m, const TreeBatchView<T>& v, T* obs, cudaStream_t s);
 };
 
 // tiles (envs) per CTA of one kernel instantiation: shared memory is the resource (one Scratch block per env).  Two
@@ -217,6 +345,43 @@ inline cudaError_t launch_tree_step(const TreeModel<T>& m, const TreeBatchView<T
   return cudaGetLastError();
 }
 
+inline int tree_knob(const char* name, int dflt) {
+  const char* e = getenv(name);
+  return e ? atoi(e) : dflt;
+}
+
+// the passes of launch_tree_step (same knobs, no env sorting) on the env kernels
+template <typename T, int LANES>
+inline cudaError_t launch_tree_env_step(const TreeModel<T>& m, const TreeBatchView<T>& v, const TreeStepArgs& a,
+                                        const TreeEnvParams<T>& env, cudaStream_t s) {
+  typedef EnvScratch<T, kFastRows, kFastCon> Fast;
+  typedef EnvScratch<T, kMaxRows, kMaxCon> Full;
+  static const int env_tiles = tree_knob("CASSIE3D_TILES", 0);
+  static const int step_barrier = tree_knob("CASSIE3D_STEP_BARRIER", 1);
+  static const int two_pass = tree_knob("CASSIE3D_TWO_PASS", 1);
+  static const int t_single = tree_tiles(k_tree_env_step<T, LANES, kMaxRows, kMaxCon, 0>, sizeof(Full), LANES, env_tiles);
+  static const int t_fast = tree_tiles(k_tree_env_step<T, LANES, kFastRows, kFastCon, 1>, sizeof(Fast), LANES, env_tiles);
+  static const int t_cont = tree_tiles(k_tree_env_step<T, LANES, kMaxRows, kMaxCon, 2>, sizeof(Full), LANES, 32 / LANES);
+  if (t_single < 0 || t_fast < 0 || t_cont < 0) return cudaErrorInvalidConfiguration;
+  TreeBatchView<T> vv = v;
+  vv.order = nullptr;
+  const T* act = (const T*)a.action;
+  const T *rq = (const T*)a.reset_q, *rv = (const T*)a.reset_qd;
+  if (!two_pass) {
+    k_tree_env_step<T, LANES, kMaxRows, kMaxCon, 0><<<(unsigned)((v.n + t_single - 1) / t_single), t_single * LANES, (size_t)t_single * sizeof(Full), s>>>(
+        m, vv, env, act, a.n_sub, a.done, rq, rv, step_barrier);
+    count_launch();
+    return cudaGetLastError();
+  }
+  k_tree_env_step<T, LANES, kFastRows, kFastCon, 1><<<(unsigned)((v.n + t_fast - 1) / t_fast), t_fast * LANES, (size_t)t_fast * sizeof(Fast), s>>>(
+      m, vv, env, act, a.n_sub, a.done, rq, rv, step_barrier);
+  count_launch();
+  k_tree_env_step<T, LANES, kMaxRows, kMaxCon, 2><<<(unsigned)((v.n + t_cont - 1) / t_cont), t_cont * LANES, (size_t)t_cont * sizeof(Full), s>>>(
+      m, vv, env, act, a.n_sub, a.done, rq, rv, 0);
+  count_launch();
+  return cudaGetLastError();
+}
+
 #define CASSIE_TREE_INSTANTIATE(T)                                                                                         \
   template <>                                                                                                              \
   cudaError_t TreeLaunch<T>::step(const TreeModel<T>& dm, const TreeBatchView<T>& v, const TreeStepArgs& a, int lanes,     \
@@ -230,6 +395,20 @@ inline cudaError_t launch_tree_step(const TreeModel<T>& m, const TreeBatchView<T
   cudaError_t TreeLaunch<T>::set_all(const TreeBatchView<T>& v, int nq, int nv, const T* q, const T* qd,                   \
                                      const uint8_t* mask, cudaStream_t s) {                                                \
     k_tree_set_all<T><<<(v.n + 127) / 128, 128, 0, s>>>(v, nq, nv, q, qd, mask);                                           \
+    count_launch();                                                                                                        \
+    return cudaGetLastError();                                                                                             \
+  }                                                                                                                        \
+  template <>                                                                                                              \
+  cudaError_t TreeLaunch<T>::env_step(const TreeModel<T>& dm, const TreeBatchView<T>& v, const TreeStepArgs& a,            \
+                                      const TreeEnvParams<T>& env, int lanes, cudaStream_t s) {                            \
+    if (lanes == 8) return launch_tree_env_step<T, 8>(dm, v, a, env, s);                                                   \
+    if (lanes == 16) return launch_tree_env_step<T, 16>(dm, v, a, env, s);                                                 \
+    if (lanes == 32) return launch_tree_env_step<T, 32>(dm, v, a, env, s);                                                 \
+    return cudaErrorInvalidValue;                                                                                          \
+  }                                                                                                                        \
+  template <>                                                                                                              \
+  cudaError_t TreeLaunch<T>::observe(const TreeModel<T>& dm, const TreeBatchView<T>& v, T* obs, cudaStream_t s) {          \
+    k_tree_observe<T><<<(v.n + kObsTiles - 1) / kObsTiles, kObsLanes * kObsTiles, 0, s>>>(dm, v, obs);                     \
     count_launch();                                                                                                        \
     return cudaGetLastError();                                                                                             \
   }

@@ -20,6 +20,8 @@ constexpr int kMaxAct = 12;
 constexpr int kMaxLevels = 12;
 constexpr int kMaxCon = 14;      // contacts kept per step (the rest are dropped and counted: mjData nconmax)
 constexpr int kMaxRows = 48;     // constraint rows per step (njmax)
+// the four foot sites of the env observation, in this order (cassie3d_stiff.xml:43-44, 86-87)
+enum FootSite { kSiteLeftFront = 0, kSiteLeftRear = 1, kSiteRightFront = 2, kSiteRightRear = 3, kNumFootSites = 4 };
 
 enum GeomType { kPlane = 0, kSphere = 2, kCapsule = 3 };
 
@@ -59,6 +61,10 @@ struct TreeModel {
   int act_dof[kMaxAct], act_limited[kMaxAct];
   T act_gear[kMaxAct], act_lo[kMaxAct], act_hi[kMaxAct];
   T qpos0[kMaxDof + 1];
+  // ---- foot contact sites (kSiteLeftFront, kSiteLeftRear, kSiteRightFront, kSiteRightRear): link and position in the
+  // link frame after welding.  Read by the env epilogue only (tree_env.cuh), so they sit behind everything the step reads.
+  int site_link[kNumFootSites];
+  T site_pos[kNumFootSites][3];
 };
 
 template <typename T, typename S>
@@ -105,6 +111,10 @@ inline void cast_tree_model(TreeModel<T>* d, const TreeModel<S>& s) {
   for (int a = 0; a < kMaxAct; a++) {
     d->act_dof[a] = s.act_dof[a]; d->act_limited[a] = s.act_limited[a];
     d->act_gear[a] = (T)s.act_gear[a]; d->act_lo[a] = (T)s.act_lo[a]; d->act_hi[a] = (T)s.act_hi[a];
+  }
+  for (int k = 0; k < kNumFootSites; k++) {
+    d->site_link[k] = s.site_link[k];
+    for (int i = 0; i < 3; i++) d->site_pos[k][i] = (T)s.site_pos[k][i];
   }
 }
 

@@ -1,4 +1,5 @@
-"""Batched 3-D Cassie (model/cassie3d_stiff.xml) on the tree engine: BASELINE.json configs[3].
+"""Batched 3-D Cassie (model/cassie3d_stiff.xml) on the tree engine: BASELINE.json configs[3], and a stand-task env on it
+(`Cassie3dBatchEnv`).
 
 The reference has no library or Python env for its 3-D model (SURVEY 8(d) config 4); this class is the batch analogue
 of the planar `Cassie2dBatch` for it: torque actions on the ten motors (cassie3d_stiff.xml:180-191), n substeps of
@@ -15,6 +16,10 @@ from . import lib as _lib
 
 # ctrlrange of the ten motors (cassie3d_stiff.xml:181-190): abduction, yaw, hip, knee, toe per leg
 TORQUE_HIGH_3D = np.array([4.5, 4.5, 12.2, 12.2, 0.9] * 2)
+# ranges of the ten actuated joints (cassie3d_stiff.xml:21-84), the PD action space [rad]
+PD_LOW_3D = np.radians([-15.0, -22.5, -50.0, -164.0, -140.0] * 2)
+PD_HIGH_3D = np.radians([22.5, 22.5, 80.0, -37.0, -30.0] * 2)
+MODE3D_BY_NAME = {"Torque": _lib.MODE3D_TORQUE, "PD": _lib.MODE3D_PD}
 
 
 def _check(rc, what):
@@ -125,3 +130,87 @@ class Cassie3dBatch:
         if self.h:
             self.L.Cassie3dBatchDestroy(self.h)
             self.h = None
+
+
+class Cassie3dBatchEnv:
+    """Stand-task env on the 3-D model (include/cassie3d.h, Cassie3dBatchEnvStep), the counterpart of the planar
+    `Cassie2dBatchEnv(task='stand')`: 45-d observation, stand reward, done 1 (fell) / 2 (diverged) / 3 (time limit),
+    auto-reset inside the step.  control_mode 'PD' (joint targets, the PD law runs at every simulator step) or 'Torque'.
+    Observation, reward and done are device tensors owned by the env and overwritten by the next call."""
+
+    def __init__(self, n_envs, device=0, control_mode="PD", precision=32, auto_reset=True, terminal_obs=False,
+                 max_path_length=0, lanes=None):
+        if control_mode not in MODE3D_BY_NAME:
+            raise ValueError("control_mode must be 'PD' or 'Torque'")
+        self.batch = Cassie3dBatch(n_envs, device, precision, lanes=lanes)
+        self.n = self.batch.n
+        self.control_mode = control_mode
+        self.mode = MODE3D_BY_NAME[control_mode]
+        self.flags = (_lib.AUTO_RESET_3D if auto_reset else 0) | (_lib.TERMINAL_OBS_3D if terminal_obs else 0)
+        self.max_path_length = int(max_path_length)
+        self.obs_dim, self.action_dim = _lib.OBS_DIM_3D, self.batch.nu
+        b = self.batch
+        self._obs = torch.empty((self.n, self.obs_dim), dtype=b.dtype, device=b.device)
+        self._rew = torch.empty(self.n, dtype=b.dtype, device=b.device)
+        self._done = torch.empty(self.n, dtype=torch.uint8, device=b.device)
+
+    @property
+    def observation_space(self):
+        high = np.full((self.obs_dim,), 1e20)
+        return -high, high
+
+    @property
+    def action_space(self):
+        if self.control_mode == "Torque":
+            return -TORQUE_HIGH_3D, TORQUE_HIGH_3D.copy()
+        return PD_LOW_3D.copy(), PD_HIGH_3D.copy()
+
+    def set_pd_gains(self, kp, kd):
+        """per-motor gains [nu] of the PD action space (default kp = 10, kd = 5)"""
+        p = np.ascontiguousarray(np.broadcast_to(np.asarray(kp, np.float64), (self.action_dim,)))
+        d = np.ascontiguousarray(np.broadcast_to(np.asarray(kd, np.float64), (self.action_dim,)))
+        dp = ct.POINTER(ct.c_double)
+        _check(self.batch.L.Cassie3dBatchSetPdGains(self.batch.h, p.ctypes.data_as(dp), d.ctypes.data_as(dp)), "SetPdGains")
+
+    def reset(self, mask=None):
+        """every env (or the masked ones) back to the reset state; returns the observation of every env"""
+        b = self.batch
+        with torch.cuda.device(b.device):
+            m = None if mask is None else mask.to(device=b.device, dtype=torch.uint8).contiguous()
+            _check(b.L.Cassie3dBatchEnvReset(b.h, None if m is None else m.data_ptr(), self._obs.data_ptr(), _stream_ptr()), "EnvReset")
+        return self._obs
+
+    def observe(self):
+        """the observation of the current state, without stepping (e.g. after batch.set_state)"""
+        b = self.batch
+        with torch.cuda.device(b.device):
+            _check(b.L.Cassie3dBatchObserve(b.h, self._obs.data_ptr(), _stream_ptr()), "Observe")
+        return self._obs
+
+    def step(self, action, n=10):
+        """n simulator steps -> obs, reward, done.  With auto_reset a done env has been reset when the call returns
+        and its obs is the reset state's (terminal_obs=True keeps the terminal one)."""
+        b = self.batch
+        a = torch.as_tensor(action, dtype=b.dtype, device=b.device).contiguous()
+        assert a.shape == (self.n, self.action_dim)
+        with torch.cuda.device(b.device):
+            _check(b.L.Cassie3dBatchEnvStep(b.h, self.mode, a.data_ptr(), int(n), self.max_path_length, self.flags,
+                                            self._obs.data_ptr(), self._rew.data_ptr(), self._done.data_ptr(),
+                                            _stream_ptr()), "EnvStep")
+        return self._obs, self._rew, self._done
+
+    def step_host(self, action_host, obs_host, reward_host, done_host, n=10):
+        """end-to-end variant: pinned host tensors in and out, copies, launches and synchronisation inside the call"""
+        b = self.batch
+        _check(b.L.Cassie3dBatchEnvStepHost(b.h, self.mode, action_host.data_ptr(), int(n), self.max_path_length, self.flags,
+                                            obs_host.data_ptr(), reward_host.data_ptr(), done_host.data_ptr()), "EnvStepHost")
+
+    def episode_lengths(self):
+        b = self.batch
+        ln = torch.empty(self.n, dtype=torch.int32, device=b.device)
+        with torch.cuda.device(b.device):
+            _check(b.L.Cassie3dBatchGetEpisodeLengths(b.h, ln.data_ptr(), _stream_ptr()), "GetEpisodeLengths")
+        return ln
+
+    def terminate(self):
+        self.batch.close()

@@ -13,6 +13,10 @@ MODE_TORQUE, MODE_PD, MODE_JACOBIAN, MODE_OSC = 0, 1, 2, 3
 TASK_STAND, TASK_IMITATE = 0, 1
 AUTO_RESET, FRESH_OBS_ON_RESET, LIVE_QSTATE, TERMINAL_OBS = 1, 2, 4, 8
 STATUS_DIVERGED = 3
+# include/cassie3d.h
+MODE3D_TORQUE, MODE3D_PD = 0, 1
+AUTO_RESET_3D, TERMINAL_OBS_3D = 1, 8
+OBS_DIM_3D = 45
 F32, F64 = 32, 64
 
 # every symbol include/cassie2d.h declares
@@ -30,7 +34,9 @@ BATCH_SYMBOLS = ["CassieGetLastError", "Cassie2dBatchInit", "Cassie2dBatchDestro
 BATCH3D_SYMBOLS = ["Cassie3dGetLastError", "Cassie3dBatchCreate", "Cassie3dBatchDestroy", "Cassie3dBatchSizes",
                    "Cassie3dBatchSetLanes", "Cassie3dBatchSetResetState", "Cassie3dBatchGetResetState", "Cassie3dBatchResetAll",
                    "Cassie3dBatchSetState", "Cassie3dBatchGetState", "Cassie3dBatchGetWarmStart", "Cassie3dBatchSetWarmStart",
-                   "Cassie3dBatchStep", "Cassie3dBatchStepHost", "Cassie3dBatchGetStats", "Cassie3dBatchGetResets"]
+                   "Cassie3dBatchStep", "Cassie3dBatchStepHost", "Cassie3dBatchGetStats", "Cassie3dBatchGetResets",
+                   "Cassie3dBatchSetPdGains", "Cassie3dBatchEnvStep", "Cassie3dBatchEnvStepHost", "Cassie3dBatchEnvReset",
+                   "Cassie3dBatchObserve", "Cassie3dBatchGetEpisodeLengths"]
 
 _lib = None
 
@@ -116,6 +122,12 @@ def load():
     L.Cassie3dBatchStepHost.argtypes = [vp, vp, ci, cd, ci, vp, vp, vp]
     L.Cassie3dBatchGetStats.argtypes = [vp, vp, vp]
     L.Cassie3dBatchGetResets.argtypes = [vp, vp, vp]
+    L.Cassie3dBatchSetPdGains.argtypes = [vp, ct.POINTER(cd), ct.POINTER(cd)]
+    L.Cassie3dBatchEnvStep.argtypes = [vp, ci, vp, ci, ci, ci, vp, vp, vp, vp]
+    L.Cassie3dBatchEnvStepHost.argtypes = [vp, ci, vp, ci, ci, ci, vp, vp, vp]
+    L.Cassie3dBatchEnvReset.argtypes = [vp, vp, vp, vp]
+    L.Cassie3dBatchObserve.argtypes = [vp, vp, vp]
+    L.Cassie3dBatchGetEpisodeLengths.argtypes = [vp, vp, vp]
     _lib = L
     return L
 

@@ -36,9 +36,9 @@ int Cassie3dBatchSetLanes(Cassie3dBatch* h, int lanes);
  * the standing pose of Cassie2d.cpp:56-58 carried over to the 3-D joints (abduction = yaw = 0) */
 int Cassie3dBatchSetResetState(Cassie3dBatch* h, const double* qpos, const double* qvel);
 int Cassie3dBatchGetResetState(Cassie3dBatch* h, double* qpos, double* qvel);
-/* every env (mask NULL) or the envs with mask[e] != 0 <- the reset state; warm start cleared */
+/* every env (mask NULL) or the envs with mask[e] != 0 <- the reset state; warm start and episode length cleared */
 int Cassie3dBatchResetAll(Cassie3dBatch* h, const uint8_t* mask, void* stream);
-/* whole-batch state I/O, real [n][nq] / [n][nv]; SetState clears the warm start */
+/* whole-batch state I/O, real [n][nq] / [n][nv]; SetState clears the warm start and the episode lengths */
 int Cassie3dBatchSetState(Cassie3dBatch* h, const void* qpos, const void* qvel, void* stream);
 int Cassie3dBatchGetState(Cassie3dBatch* h, void* qpos, void* qvel, void* stream);
 int Cassie3dBatchGetWarmStart(Cassie3dBatch* h, void* qacc_warmstart, void* stream);
@@ -56,6 +56,44 @@ int Cassie3dBatchStepHost(Cassie3dBatch* h, const void* action, int n_substeps, 
 int Cassie3dBatchGetStats(Cassie3dBatch* h, int32_t* stats, void* stream);
 /* int32 [n]: auto-resets so far */
 int Cassie3dBatchGetResets(Cassie3dBatch* h, int32_t* resets, void* stream);
+
+/* ---- stand-task environment (the planar Cassie2dBatchEnvStep's counterpart; the 3-D model has no reference env, so the
+ * task is a design carried over from rllab/envs/cassie_stand2d.py:119-133, DESIGN.md section 11).
+ *
+ * action real [n][nu], motors in file order (abduction, yaw, hip, knee, toe per leg, left leg first):
+ *   CASSIE3D_MODE_TORQUE  the controls, held for the n_substeps simulator steps (clamped to ctrlrange)
+ *   CASSIE3D_MODE_PD      joint targets [rad]; before EVERY simulator step u = kp (target - q) - kd qd on each motor's
+ *                         joint, then clamped to ctrlrange.  Gains per handle, default kp = 10, kd = 5 (Cassie2d.cpp:96-112)
+ * obs real [n][CASSIE3D_OBS_DIM] of the state after the last simulator step: [0] pelvis height, [1..4] pelvis quaternion
+ *   w x y z, [5..18] the 14 hinge angles, [19..38] qvel (linear velocity in world axes, angular velocity in pelvis axes,
+ *   hinge rates), [39..41] left and [42..44] right foot minus pelvis position in world axes (a foot is the mean of its
+ *   *_contact_front and *_contact_rear sites)
+ * reward real [n] = 1 - 2 (0.9 - z)^2 - 2 |c|^2 - 0.001 |action|^2, z = pelvis height, c = horizontal offset of the feet
+ *   midpoint from the pelvis; 0 for a diverged env
+ * done uint8 [n]: 2 the state is not finite or beyond 1e10 (the env is then always reset), else 1 pelvis below 0.5 m,
+ *   else 3 the episode length reached max_path_length > 0, else 0
+ * flags: CASSIE3D_AUTO_RESET: done envs restart from the reset state inside the call (warm start cleared), and the
+ *   observation returned is the reset state's unless CASSIE3D_TERMINAL_OBS asks for the terminal one (a diverged env
+ *   always returns the reset state's).  Episode length: +1 per EnvStep, 0 after every reset (EnvReset, ResetAll,
+ *   SetState, auto-reset). */
+enum { CASSIE3D_MODE_TORQUE = 0, CASSIE3D_MODE_PD = 1 };
+enum { CASSIE3D_AUTO_RESET = 1, CASSIE3D_TERMINAL_OBS = 8 };
+enum { CASSIE3D_OBS_DIM = 45 };
+/* host doubles, [nu] each */
+int Cassie3dBatchSetPdGains(Cassie3dBatch* h, const double* kp, const double* kd);
+/* n_substeps >= 1 simulator steps of every env, then observation, reward, done; obs / reward / done are required */
+int Cassie3dBatchEnvStep(Cassie3dBatch* h, int mode, const void* action, int n_substeps, int max_path_length, int flags,
+                         void* obs, void* reward, uint8_t* done, void* stream);
+/* the same with HOST buffers: action in, obs / reward / done out (each may be NULL); copies and the synchronisation are
+ * inside the call */
+int Cassie3dBatchEnvStepHost(Cassie3dBatch* h, int mode, const void* action, int n_substeps, int max_path_length, int flags,
+                             void* obs, void* reward, uint8_t* done);
+/* ResetAll(mask) (NULL = every env), then the observation of EVERY env into obs (obs may be NULL) */
+int Cassie3dBatchEnvReset(Cassie3dBatch* h, const uint8_t* mask, void* obs, void* stream);
+/* the observation of the current state of every env, without stepping (e.g. after SetState) */
+int Cassie3dBatchObserve(Cassie3dBatch* h, void* obs, void* stream);
+/* int32 [n]: EnvStep calls since each env's last reset */
+int Cassie3dBatchGetEpisodeLengths(Cassie3dBatch* h, int32_t* ep_len, void* stream);
 
 #ifdef __cplusplus
 }

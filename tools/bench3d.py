@@ -4,6 +4,10 @@ on the ten motors held 10 simulator steps, done when the pelvis drops below 0.5 
 bench.py's format (value, e2e, roofline, cpu_baseline, clocks).  Not the headline bench (that is bench.py, configs[2]).
 
   python tools/bench3d.py [--envs 8192] [--steps 20] [--warmup 3] [--lanes 32]       (under torchrun for N > 1 GPUs)
+
+--workload env_torque: the same torques through Cassie3dBatchEnvStep (observation, reward, done, time limit 1000 policy
+steps: what the stand env's epilogue costs); env_pd: uniform-random PD targets within the joint ranges, auto-reset,
+max_path_length 1000.  Device-timed and end-to-end (EnvStepHost: obs / reward / done to the host) env-steps/s.
 """
 import argparse
 import json
@@ -27,12 +31,13 @@ p.add_argument("--precision", type=int, default=32)
 p.add_argument("--preadvance", type=int, default=2000, help="simulator steps before timing: robots fall after ~1000 steps of random torques and reset, by 2000 the batch is a mix of phases")
 p.add_argument("--no-cpu-baseline", action="store_true")
 p.add_argument("--cpu-seconds", type=float, default=10.0)
+p.add_argument("--workload", choices=["torque", "env_torque", "env_pd"], default="torque")
 a = p.parse_args()
 
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 from cassierl_b200 import lib  # noqa: E402
-from cassierl_b200.envs3d import Cassie3dBatch, TORQUE_HIGH_3D  # noqa: E402
+from cassierl_b200.envs3d import PD_HIGH_3D, PD_LOW_3D, TORQUE_HIGH_3D, Cassie3dBatch, Cassie3dBatchEnv  # noqa: E402
 
 world = int(os.environ.get("WORLD_SIZE", "1")); rank = int(os.environ.get("RANK", "0")); local = int(os.environ.get("LOCAL_RANK", "0"))
 torch.cuda.set_device(local)
@@ -43,13 +48,35 @@ L = lib.load()
 n, sub = a.envs, a.substeps
 dt_t = torch.float64 if a.precision == 64 else torch.float32
 rs = 8 if a.precision == 64 else 4
-b = Cassie3dBatch(n, device=local, precision=a.precision, lanes=a.lanes or None)
+ENV = a.workload != "torque"
+MPL = 1000
+
+
+def make():
+    if ENV:
+        return Cassie3dBatchEnv(n, device=local, control_mode="PD" if a.workload == "env_pd" else "Torque", precision=a.precision,
+                                max_path_length=MPL, lanes=a.lanes or None)
+    return Cassie3dBatch(n, device=local, precision=a.precision, lanes=a.lanes or None)
+
+
+e3 = make()
+b = e3.batch if ENV else e3
 n_pre = (a.preadvance + sub - 1) // sub
 total = n_pre + a.warmup + a.steps
 gen = torch.Generator(device=dev).manual_seed(1 + rank)
 hi = torch.tensor(TORQUE_HIGH_3D, dtype=dt_t, device=dev)
 acts = (torch.rand((total, n, 10), generator=gen, device=dev, dtype=dt_t) * 2 - 1) * hi     # resident in HBM before timing
+if a.workload == "env_pd":    # uniform within the joint ranges
+    lo = torch.tensor(PD_LOW_3D, dtype=dt_t, device=dev); span = torch.tensor(PD_HIGH_3D, dtype=dt_t, device=dev) - lo
+    acts = lo + torch.rand((total, n, 10), generator=gen, device=dev, dtype=dt_t) * span
 done = torch.empty(n, dtype=torch.uint8, device=dev)
+
+
+def step(h, act):
+    if ENV:
+        h.step(act, n=sub)
+    else:
+        h.step(act, n=sub, z_done=0.5, auto_reset=True, done=done)
 flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
 
 
@@ -60,7 +87,7 @@ def barrier():
 
 
 for k in range(n_pre + a.warmup):
-    b.step(acts[k], n=sub, z_done=0.5, auto_reset=True, done=done)
+    step(e3, acts[k])
 barrier()
 sampler = bench.ClockSampler(local, "GPU-" + str(torch.cuda.get_device_properties(dev).uuid))
 if rank == 0:
@@ -72,7 +99,7 @@ barrier()
 for k in range(a.steps):
     flush.zero_()
     ev[k][0].record()
-    b.step(acts[n_pre + a.warmup + k], n=sub, z_done=0.5, auto_reset=True, done=done)
+    step(e3, acts[n_pre + a.warmup + k])
     ev[k][1].record()
 barrier()
 launches = L.CassieKernelLaunchCount() - l0
@@ -90,19 +117,30 @@ stats = torch.stack([st[:, 0].mean(), st[:, 1].mean(), st[:, 2].mean(), st[:, 3]
 if world > 1:
     red = stats.clone(); dist.all_reduce(red); stats[3:] = red[3:]
 
-# end to end: pinned host actions in, qpos / qvel / done out, copies inside the timed region
-b2 = Cassie3dBatch(n, device=local, precision=a.precision, lanes=a.lanes or None)
+# end to end: pinned host actions in, qpos / qvel / done out (env workloads: obs / reward / done), copies inside the
+# timed region
+b2 = make()
 for k in range(n_pre):
-    b2.step(acts[k], n=sub, z_done=0.5, auto_reset=True, done=done)
+    step(b2, acts[k])
 acts_h = acts[n_pre:].cpu().pin_memory()
 qh = torch.empty((n, 21), dtype=dt_t).pin_memory(); vh = torch.empty((n, 20), dtype=dt_t).pin_memory()
 dh = torch.empty(n, dtype=torch.uint8).pin_memory()
+oh = torch.empty((n, 45), dtype=dt_t).pin_memory(); rh = torch.empty(n, dtype=dt_t).pin_memory()
+
+
+def step_host(act_h):
+    if ENV:
+        b2.step_host(act_h, oh, rh, dh, n=sub)
+    else:
+        b2.step_host(act_h, qh, vh, dh, n=sub, z_done=0.5, auto_reset=True)
+
+
 for k in range(a.warmup):
-    b2.step_host(acts_h[k], qh, vh, dh, n=sub, z_done=0.5, auto_reset=True)
+    step_host(acts_h[k])
 barrier()
 t0 = time.perf_counter()
 for k in range(a.steps):
-    b2.step_host(acts_h[a.warmup + k], qh, vh, dh, n=sub, z_done=0.5, auto_reset=True)
+    step_host(acts_h[a.warmup + k])
 torch.cuda.synchronize()
 el = torch.tensor([time.perf_counter() - t0], dtype=torch.float64, device=dev)
 if world > 1:
@@ -151,6 +189,13 @@ if rank == 0:
             "gpu_launches": int(launches), "clocks": clocks,
             "stats": {"rows_mean": float(stats[0]), "contacts_mean": float(stats[1]), "pgs_sweeps_mean": float(stats[2]), "contacts_dropped": int(stats[3]),
                       "auto_resets_in_timed_region": int(stats[4]), "non_finite_envs": int(stats[5]), "smem_bytes_per_env": b.smem_per_env}}
+    if ENV:
+        line["metric"] = "env-steps/sec cassie3d_stiff stand env (%s), EnvStep with observation, reward, auto-reset" % a.workload
+        line["config"]["workload"] = ("%s actions held %d sim steps through Cassie3dBatchEnvStep: 45-d observation, stand reward, done at "
+                                      "pelvis z < 0.5 m or after %d policy steps, auto-reset" %
+                                      ("uniform-random torques" if a.workload == "env_torque" else "uniform-random PD targets within the joint ranges", sub, MPL))
+        line["config"]["bench_workload"] = a.workload
+        line["e2e"]["d2h_bytes_per_step"] = n * (46 * rs + 1)
     if not a.no_cpu_baseline and world == 1:
         from oracle import oracle as O
         O.build()
