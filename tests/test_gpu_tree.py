@@ -76,7 +76,7 @@ def test_tree_fp64_fall_and_autoreset_bit_exact(oracle, omodel3d):
     assert _err(q, v, qo, vo).max() < 1e-8
 
 
-@pytest.mark.parametrize("lanes", [8, 32])
+@pytest.mark.parametrize("lanes", [8, 16, 32])
 def test_tree_fp32_single_step_vs_oracle(oracle, omodel3d, lanes):
     """fp32 build, teacher-forced: every step starts from the oracle's state and warm start.  1e-5 on the steps whose
     constraint-row count equals the oracle's; event mismatches (a contact within fp32 rounding of touching) are rare"""
