@@ -30,7 +30,8 @@ def _deps(unit=None):
     if unit and (unit.startswith("kernels_") or unit.startswith("rollout_")):
         names = [f for f in names if f == unit or (f.endswith((".cuh", ".h")) and not f.startswith(("tree_", "cassie3d", "mjcf_flatten")))]
     elif unit and (unit.startswith("tree_") or unit.startswith("cassie3d")):
-        names = [f for f in names if f == unit or f.startswith("tree_") and f.endswith((".cuh", ".h")) or f == "mjcf_flatten.h"]
+        shared = ("mjcf_flatten.h", "rollout_philox.cuh", "rollout_args.h")   # the 3-D rollout's noise and sampler launches
+        names = [f for f in names if f == unit or f.startswith("tree_") and f.endswith((".cuh", ".h")) or f in shared]
     inc = ("cassie3d.h",) if unit and (unit.startswith("tree_") or unit.startswith("cassie3d")) else ("cassie2d.h",)
     return [os.path.join(CSRC, f) for f in names] + [os.path.join(HERE, "..", "include", h) for h in inc]
 

@@ -8,6 +8,7 @@
 
 #include "../../include/cassie3d.h"
 #include "mjcf_flatten.h"
+#include "rollout_args.h"
 #include "tree_kernels.cuh"
 
 using namespace cassie;
@@ -55,6 +56,8 @@ struct Cassie3dBatch {
   void* d_obs = nullptr;      // host-variant staging of EnvStepHost
   void* d_reward = nullptr;
   int32_t* ep_len = nullptr;  // [n] policy steps since the env's last reset (EnvStep)
+  int32_t* policy_step = nullptr;   // [n] Philox step counter of Rollout: zero at Create, advanced by Rollout only
+  void* d_act_env = nullptr;  // [n][nu] the mapped, clipped action of Rollout's current policy step
   std::vector<double> kp, kd; // PD gains of the env's kActPd action space, per motor
   cudaStream_t own_stream = nullptr;
   size_t rs() const { return precision == 64 ? 8 : 4; }
@@ -88,7 +91,8 @@ int setup(Cassie3dBatch* h, TreeBatchView<T>& v) {
       dmalloc(h, (void**)&v.resume, sizeof(int32_t) * n) || dmalloc(h, &h->d_reset_q, sizeof(T) * m.nq) ||
       dmalloc(h, &h->d_reset_qd, sizeof(T) * m.nv) || dmalloc(h, &h->d_action, sizeof(T) * n * m.nu) ||
       dmalloc(h, (void**)&h->d_done, n) || dmalloc(h, &h->d_obs, sizeof(T) * n * kObsDim3d) ||
-      dmalloc(h, &h->d_reward, sizeof(T) * n) || dmalloc(h, (void**)&h->ep_len, sizeof(int32_t) * n))
+      dmalloc(h, &h->d_reward, sizeof(T) * n) || dmalloc(h, (void**)&h->ep_len, sizeof(int32_t) * n) ||
+      dmalloc(h, (void**)&h->policy_step, sizeof(int32_t) * n) || dmalloc(h, &h->d_act_env, sizeof(T) * n * m.nu))
     return -1;
   return 0;
 }
@@ -135,6 +139,38 @@ int env_step(Cassie3dBatch* h, int mode, const void* action, int n_sub, int max_
 }
 
 template <typename T>
+int rollout(Cassie3dBatch* h, int mode, const void* params, int T_steps, int n_sub, int max_path_length, int normalize,
+            unsigned long long seed, unsigned int env0, void* obs, void* act, void* mean, void* reward, uint8_t* done,
+            cudaStream_t s) {
+  const size_t n = (size_t)h->n, nu = (size_t)h->model.nu;
+  TreeStepArgs a;
+  a.action = nullptr; a.n_sub = n_sub; a.z_done = 0; a.auto_reset = 1; a.done = nullptr;
+  a.reset_q = h->d_reset_q; a.reset_qd = h->d_reset_qd;
+  TreeEnvParams<T> ep;
+  for (int i = 0; i < kMaxAct; i++) {
+    ep.kp[i] = i < h->model.nu ? (T)h->kp[i] : (T)0;
+    ep.kd[i] = i < h->model.nu ? (T)h->kd[i] : (T)0;
+  }
+  ep.mode = mode; ep.flags = kEnvAutoReset; ep.max_path_length = max_path_length;
+  ep.obs = nullptr; ep.reward = nullptr; ep.ep_len = h->ep_len;
+  TreeRolloutParams<T> ro;
+  double lo[kMaxAct] = {0}, hi[kMaxAct] = {0};
+  action_box(h->model, mode, lo, hi);
+  for (int i = 0; i < kMaxAct; i++) { ro.lo[i] = (T)lo[i]; ro.hi[i] = (T)hi[i]; }
+  ro.params = (const T*)params; ro.normalize = normalize; ro.seed = seed; ro.env0 = env0;
+  ro.policy_step = h->policy_step; ro.act_env = (T*)h->d_act_env;
+  for (int k = 0; k < T_steps; k++) {   // one launch pass per policy step, no host synchronisation in between
+    ro.obs = (T*)obs + (size_t)k * n * kObsDim3d;
+    ro.act = (T*)act + (size_t)k * n * nu;
+    ro.mean = (T*)mean + (size_t)k * n * nu;
+    ro.rew = (T*)reward + (size_t)k * n;
+    ro.done = done + (size_t)k * n;
+    CU3_OK(TreeLaunch<T>::rollout_step(model_of<T>(h), view<T>(h), a, ep, ro, h->lanes, s));
+  }
+  return 0;
+}
+
+template <typename T>
 int observe(Cassie3dBatch* h, void* obs, cudaStream_t s) {
   CU3_OK(TreeLaunch<T>::observe(model_of<T>(h), view<T>(h), (T*)obs, s));
   return 0;
@@ -153,6 +189,8 @@ int check_env_step(Cassie3dBatch* h, int mode, const void* action, int n_substep
 static_assert((int)CASSIE3D_MODE_TORQUE == (int)kActTorque && (int)CASSIE3D_MODE_PD == (int)kActPd, "action modes");
 static_assert((int)CASSIE3D_AUTO_RESET == (int)kEnvAutoReset && (int)CASSIE3D_TERMINAL_OBS == (int)kEnvTerminalObs, "env flags");
 static_assert((int)CASSIE3D_OBS_DIM == kObsDim3d, "observation size");
+static_assert((int)CASSIE3D_POLICY_PARAMS == kPolicyParams3d, "policy parameter count");
+static_assert(kMaxFeat3d == 2 * kObsDim3d + 4, "baseline features of the 3-D observation");
 
 #define DISPATCH3(h, expr32, expr64) ((h)->precision == 64 ? (expr64) : (expr32))
 
@@ -382,6 +420,75 @@ int Cassie3dBatchObserve(Cassie3dBatch* h, void* obs, void* stream) {
   DeviceGuard g(h->device);
   cudaStream_t s = (cudaStream_t)stream;
   return DISPATCH3(h, observe<float>(h, obs, s), observe<double>(h, obs, s));
+}
+
+int Cassie3dBatchRollout(Cassie3dBatch* h, int mode, const void* params_dev, int n_params, int n_policy_steps,
+                         int n_substeps, int max_path_length, int normalize, unsigned long long seed,
+                         unsigned int first_global_env, void* obs_dev, void* action_dev, void* mean_dev,
+                         void* reward_dev, uint8_t* done_dev, void* stream) {
+  if (!h || !params_dev || !obs_dev || !action_dev || !mean_dev || !reward_dev || !done_dev) return fail3("null argument");
+  if (mode != CASSIE3D_MODE_TORQUE && mode != CASSIE3D_MODE_PD) return fail3("mode must be CASSIE3D_MODE_TORQUE or CASSIE3D_MODE_PD");
+  if (n_policy_steps < 0) return fail3("n_policy_steps must not be negative");
+  if (n_substeps < 1) return fail3("n_substeps must be at least 1");
+  if (max_path_length <= 0) return fail3("max_path_length must be positive");
+  if (n_params != kPolicyParams3d)
+    return fail3("policy parameter vector has " + std::to_string(n_params) + " entries, expected " + std::to_string(kPolicyParams3d));
+  if (h->model.nu != kPolicyAct3d) return fail3("the policy has " + std::to_string(kPolicyAct3d) + " actions, the model " + std::to_string(h->model.nu) + " motors");
+  DeviceGuard g(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  return DISPATCH3(h, rollout<float>(h, mode, params_dev, n_policy_steps, n_substeps, max_path_length, normalize, seed,
+                                     first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s),
+                   rollout<double>(h, mode, params_dev, n_policy_steps, n_substeps, max_path_length, normalize, seed,
+                                   first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s));
+}
+
+int Cassie3dBatchActionBox(Cassie3dBatch* h, int mode, double* lo, double* hi) {
+  if (!h || !lo || !hi) return fail3("null argument");
+  if (mode != CASSIE3D_MODE_TORQUE && mode != CASSIE3D_MODE_PD) return fail3("mode must be CASSIE3D_MODE_TORQUE or CASSIE3D_MODE_PD");
+  action_box(h->model, mode, lo, hi);
+  return 0;
+}
+
+int Cassie3dBatchDiscountedReturns(Cassie3dBatch* h, const void* reward_dev, const uint8_t* done_dev, const void* tail_dev,
+                                   double gamma, int n_policy_steps, void* returns_dev, void* stream) {
+  if (!h || !reward_dev || !done_dev || !returns_dev) return fail3("null argument");
+  if (n_policy_steps < 0) return fail3("n_policy_steps must not be negative");
+  DeviceGuard g(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (h->precision == 64) CU3_OK(launch_discounted_returns<double>(reward_dev, done_dev, tail_dev, gamma, n_policy_steps, h->n, returns_dev, s));
+  else CU3_OK(launch_discounted_returns<float>(reward_dev, done_dev, tail_dev, gamma, n_policy_steps, h->n, returns_dev, s));
+  return 0;
+}
+
+int Cassie3dBatchBaselineMoments(Cassie3dBatch* h, const void* obs_dev, const void* returns_dev, const uint8_t* done_dev,
+                                 const int32_t* path_start_dev, int n_policy_steps, int32_t* path_index_dev,
+                                 double* moments_dev, void* stream) {
+  if (!h || !obs_dev || !returns_dev || !done_dev || !path_index_dev || !moments_dev) return fail3("null argument");
+  if (n_policy_steps < 0) return fail3("n_policy_steps must not be negative");
+  DeviceGuard g(h->device);
+  BaselineArgs a{};
+  a.obs = obs_dev; a.ret = returns_dev; a.done = done_dev; a.start = path_start_dev; a.idx = path_index_dev; a.moments = moments_dev;
+  a.odim = kObsDim3d; a.T_steps = n_policy_steps; a.n = h->n;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (h->precision == 64) CU3_OK((launch_baseline_moments<double, kMaxFeat3d, kMomentsPerThread3d>(a, s)));
+  else CU3_OK((launch_baseline_moments<float, kMaxFeat3d, kMomentsPerThread3d>(a, s)));
+  return 0;
+}
+
+int Cassie3dBatchAdvantages(Cassie3dBatch* h, const void* obs_dev, const void* reward_dev, const uint8_t* done_dev,
+                            const int32_t* path_index_dev, const void* coeffs_dev, double gamma, double gae_lambda,
+                            int n_policy_steps, void* advantages_dev, void* values_dev, void* stream) {
+  if (!h || !obs_dev || !reward_dev || !done_dev || !path_index_dev || !coeffs_dev || !advantages_dev) return fail3("null argument");
+  if (n_policy_steps < 0) return fail3("n_policy_steps must not be negative");
+  DeviceGuard g(h->device);
+  BaselineArgs a{};
+  a.obs = obs_dev; a.rew = reward_dev; a.done = done_dev; a.idx = const_cast<int32_t*>(path_index_dev); a.coeffs = coeffs_dev;
+  a.adv = advantages_dev; a.value = values_dev; a.odim = kObsDim3d; a.T_steps = n_policy_steps; a.n = h->n;
+  a.gamma = gamma; a.lambda = gae_lambda;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (h->precision == 64) CU3_OK((launch_advantages<double, kMaxFeat3d>(a, s)));
+  else CU3_OK((launch_advantages<float, kMaxFeat3d>(a, s)));
+  return 0;
 }
 
 int Cassie3dBatchGetEpisodeLengths(Cassie3dBatch* h, int32_t* ep_len, void* stream) {

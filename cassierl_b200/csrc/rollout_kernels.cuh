@@ -11,6 +11,7 @@
 // results do not depend on the launch partition or the GPU count.
 #pragma once
 #include "env_kernels.cuh"
+#include "rollout_philox.cuh"
 #include "rollout_args.h"
 #include <cstdlib>
 #include <cstring>
@@ -18,36 +19,6 @@
 namespace cassie {
 
 constexpr int kHidden = 32;  // hidden_sizes=(32, 32), trpo_cassie.py:24
-
-// ---- Philox4x32-10 (Salmon et al., SC'11), counter-based
-__host__ __device__ inline void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
-  for (int r = 0; r < 10; r++) {
-    const uint64_t p0 = (uint64_t)0xD2511F53u * c[0], p1 = (uint64_t)0xCD9E8D57u * c[2];
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0, n1 = (uint32_t)p1;
-    const uint32_t n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1, n3 = (uint32_t)p0;
-    c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
-    k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-  }
-}
-// eight standard normals for (seed, env, step): two Philox blocks, Box-Muller on (0,1] uniforms
-template <typename T>
-__device__ inline void normal8(uint64_t seed, uint32_t env, uint32_t step, T out[8]) {
-#pragma unroll
-  for (int b = 0; b < 2; b++) {
-    uint32_t c[4] = {env, step, (uint32_t)b, 0u};
-    philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
-#pragma unroll
-    for (int p = 0; p < 2; p++) {
-      const float u1 = ((float)(c[2 * p] >> 8) + 1.0f) * (1.0f / 16777216.0f);   // (0, 1]
-      const float u2 = (float)(c[2 * p + 1] >> 8) * (1.0f / 16777216.0f);        // [0, 1)
-      const float rad = sqrtf(-2.0f * logf(u1));
-      float sn, cs;
-      sincospif(2.0f * u2, &sn, &cs);
-      out[4 * b + 2 * p] = (T)(rad * cs);
-      out[4 * b + 2 * p + 1] = (T)(rad * sn);
-    }
-  }
-}
 
 // ---- tensor-core variant of the policy forward (A/B of VERDICT r1 item 8; CASSIE_MLP=tc, fp32 builds, thread engine)
 // One warp = 32 envs = the M dimension: H[32 x 32] = X[32 x K] W[K x 32] as mma.sync m16n8k8 TF32 tiles, every product
@@ -313,7 +284,8 @@ cudaError_t launch_discounted_returns(const void* rew, const uint8_t* done, cons
 // normal equations F'F (D x D) and F'y (D) over all T x n samples (the D x D solve itself is host-side
 // glue on 38 x 38 numbers); k_advantages evaluates the baseline and runs the backward GAE scan
 //   delta_t = r_t + gamma V_{t+1} - V_t,  A_t = delta_t + gamma lambda A_{t+1}   (V = 0 past a path end).
-constexpr int kMaxFeat = 2 * 26 + 4;
+// The capacities are template parameters: the planar observations below, the 3-D one in rollout_args.h.
+constexpr int kMaxFeat = 2 * 26 + 4, kMomentsPerThread = 8;
 
 template <typename T>
 __device__ __forceinline__ void baseline_features(const T* __restrict__ o, int odim, int step_in_path, T* f) {
@@ -341,16 +313,17 @@ __global__ void __launch_bounds__(128) k_path_index(const uint8_t* __restrict__ 
 }
 
 // one CTA per chunk of samples: features staged in shared memory, thread p owns entries p, p + 256, ... of
-// the packed upper triangle (+ the F'y column); double accumulation, one atomicAdd per entry per CTA
-template <typename T>
+// the packed upper triangle (+ the F'y column); double accumulation, one atomicAdd per entry per CTA.
+// MAXF = feature capacity (D <= MAXF), EPT = entries per thread (D (D + 1) / 2 + D <= 256 EPT).
+template <typename T, int MAXF, int EPT>
 __global__ void __launch_bounds__(256) k_baseline_moments(const T* __restrict__ obs, const T* __restrict__ ret,
                                                           const int32_t* __restrict__ idx, int odim, long n_samples,
                                                           int chunk, double* __restrict__ out) {
   const int D = 2 * odim + 4, n_ent = D * (D + 1) / 2 + D;
-  __shared__ T sf[32][kMaxFeat + 1];
-  double acc[8];
+  __shared__ T sf[32][MAXF + 1];
+  double acc[EPT];
 #pragma unroll
-  for (int q = 0; q < 8; q++) acc[q] = 0.0;
+  for (int q = 0; q < EPT; q++) acc[q] = 0.0;
   const long s0 = (long)blockIdx.x * chunk, s1 = s0 + chunk < n_samples ? s0 + chunk : n_samples;
   for (long base = s0; base < s1; base += 32) {
     const int cnt = (int)(s1 - base < 32 ? s1 - base : 32);
@@ -362,7 +335,7 @@ __global__ void __launch_bounds__(256) k_baseline_moments(const T* __restrict__ 
     }
     __syncthreads();
 #pragma unroll
-    for (int q = 0; q < 8; q++) {
+    for (int q = 0; q < EPT; q++) {
       const int p = threadIdx.x + 256 * q;
       if (p < n_ent) {
         int i, j;  // entry p -> (i, j): packed rows of the upper triangle, then the F'y column (j = D)
@@ -378,13 +351,13 @@ __global__ void __launch_bounds__(256) k_baseline_moments(const T* __restrict__ 
     }
   }
 #pragma unroll
-  for (int q = 0; q < 8; q++) {
+  for (int q = 0; q < EPT; q++) {
     const int p = threadIdx.x + 256 * q;
     if (p < n_ent) atomicAdd(out + p, acc[q]);
   }
 }
 
-template <typename T>
+template <typename T, int MAXF>
 __global__ void __launch_bounds__(128) k_advantages(const T* __restrict__ obs, const T* __restrict__ rew,
                                                     const uint8_t* __restrict__ done, const int32_t* __restrict__ idx,
                                                     const T* __restrict__ coeffs, int odim, T gamma, T lambda, int T_steps, int n,
@@ -392,7 +365,7 @@ __global__ void __launch_bounds__(128) k_advantages(const T* __restrict__ obs, c
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= n) return;
   const int D = 2 * odim + 4;
-  T f[kMaxFeat];
+  T f[MAXF];
   T v_next = T(0), a_next = T(0);
   for (int t = T_steps - 1; t >= 0; t--) {
     const size_t i = (size_t)t * n + e;
@@ -408,7 +381,7 @@ __global__ void __launch_bounds__(128) k_advantages(const T* __restrict__ obs, c
   }
 }
 
-template <typename T>
+template <typename T, int MAXF, int EPT>
 cudaError_t launch_baseline_moments(const BaselineArgs& a, cudaStream_t s) {
   k_path_index<T><<<grid_for(a.n, 128), 128, 0, s>>>(a.done, a.T_steps, a.n, a.start, a.idx);
   const long n_samples = (long)a.T_steps * a.n;
@@ -416,17 +389,26 @@ cudaError_t launch_baseline_moments(const BaselineArgs& a, cudaStream_t s) {
   const int D = 2 * a.odim + 4;
   cudaError_t e = cudaMemsetAsync(a.moments, 0, sizeof(double) * (D * (D + 1) / 2 + D), s);
   if (e != cudaSuccess) return e;
-  k_baseline_moments<T><<<(unsigned)((n_samples + chunk - 1) / chunk), 256, 0, s>>>((const T*)a.obs, (const T*)a.ret, a.idx, a.odim,
+  k_baseline_moments<T, MAXF, EPT><<<(unsigned)((n_samples + chunk - 1) / chunk), 256, 0, s>>>((const T*)a.obs, (const T*)a.ret, a.idx, a.odim,
                                                                                   n_samples, chunk, a.moments);
   count_launch(); count_launch();
   return cudaGetLastError();
 }
-template <typename T>
+template <typename T, int MAXF>
 cudaError_t launch_advantages(const BaselineArgs& a, cudaStream_t s) {
-  k_advantages<T><<<grid_for(a.n, 128), 128, 0, s>>>((const T*)a.obs, (const T*)a.rew, a.done, a.idx, (const T*)a.coeffs, a.odim,
+  k_advantages<T, MAXF><<<grid_for(a.n, 128), 128, 0, s>>>((const T*)a.obs, (const T*)a.rew, a.done, a.idx, (const T*)a.coeffs, a.odim,
                                                     (T)a.gamma, (T)a.lambda, a.T_steps, a.n, (T*)a.adv, (T*)a.value);
   count_launch();
   return cudaGetLastError();
+}
+// the planar observations (batch_state.h)
+template <typename T>
+cudaError_t launch_baseline_moments(const BaselineArgs& a, cudaStream_t s) {
+  return launch_baseline_moments<T, kMaxFeat, kMomentsPerThread>(a, s);
+}
+template <typename T>
+cudaError_t launch_advantages(const BaselineArgs& a, cudaStream_t s) {
+  return launch_advantages<T, kMaxFeat>(a, s);
 }
 
 template <typename T>

@@ -109,6 +109,12 @@ TREE_FN void load_reset(const Tile<LANES>& tl, const TreeModel<T>& m, SC& s, con
   tl.sync();
 }
 
+// the env kernels' per-env scratch: the step's, plus the action as given (PD targets survive all substeps in it)
+template <typename T, int ROWS = kMaxRows, int CON = kMaxCon>
+struct EnvScratch : Scratch<T, ROWS, CON> {
+  T target[kMaxAct];
+};
+
 struct EnvResult { int done, len; bool reset; };
 
 // The epilogue of one env after the last substep of an EnvStep: reward (every lane holds it), done code, episode length

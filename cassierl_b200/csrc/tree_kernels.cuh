@@ -6,8 +6,10 @@
 #include <cstdint>
 #include <cstdlib>
 #include <cuda_runtime.h>
+#include "rollout_philox.cuh"
 #include "tree_engine.cuh"
 #include "tree_env.cuh"
+#include "tree_rollout.cuh"
 
 namespace cassie {
 void count_launch();
@@ -133,12 +135,6 @@ struct TreeEnvParams {
   int32_t* ep_len;              // [n] policy steps since the env's last reset
 };
 
-// the env kernels' per-env scratch: the step's, plus the action as given (PD targets survive all substeps in it)
-template <typename T, int ROWS, int CON>
-struct EnvScratch : Scratch<T, ROWS, CON> {
-  T target[kMaxAct];
-};
-
 // Cassie3dBatchEnvStep: the passes of k_tree_step (same MODEs, same physics) with the env's action space -- in kActPd the
 // PD law runs ahead of every substep on the targets kept in s.target, which the continuation pass re-reads from `action`
 // -- and, instead of the z_done rule, the stand task's epilogue (tree_env.cuh).  The epilogue runs in the pass that
@@ -200,6 +196,112 @@ k_tree_env_step(const __grid_constant__ TreeModel<T> m, const TreeBatchView<T> v
     if (MODE != 0) v.resume[e] = k_done;
     if (alive) {
       done[e] = (uint8_t)r.done;
+      if (n_sub > k0) {
+        v.stats[4 * e + 0] = st.nefc; v.stats[4 * e + 1] = st.ncon; v.stats[4 * e + 2] = st.sweeps;
+        v.stats[4 * e + 3] += st.dropped;
+      }
+      if (r.reset) v.resets[e] += 1;
+    }
+  }
+}
+
+// What the rollout variant of the env kernel (k_tree_rollout_step, Cassie3dBatchRollout) adds: the policy, the noise
+// keys, the action box and the path buffers of ONE policy step (the host offsets them to row k of the [T][n][.] buffers).
+template <typename T>
+struct TreeRolloutParams {
+  T lo[kMaxAct], hi[kMaxAct];   // action box: ctrlrange (torque mode) or the motors' joint ranges (PD mode)
+  const T* params;              // [kPolicyParams3d] GaussianMLPPolicy.flat
+  int normalize;                // NormalizedEnv's affine map before the clip
+  uint64_t seed;
+  uint32_t env0;                // global id of this batch's env 0
+  int32_t* policy_step;         // [n] Philox step counter, advanced by every finished policy step
+  T* act_env;                   // [n][nu] the mapped, clipped action (the continuation pass reads it)
+  T* obs;                       // [n][kObsDim3d] row k: the observation the policy saw
+  T* act;                       // [n][nu] raw policy output
+  T* mean;                      // [n][nu]
+  T* rew;                       // [n]
+  uint8_t* done;                // [n] path codes: 1 terminated, 2 cut at max_path_length
+};
+
+// One policy step of Cassie3dBatchRollout: the passes of k_tree_env_step (same MODEs, physics and stand-task epilogue,
+// auto-reset always on), with the policy's prologue (tree_rollout.cuh) in MODE 0 / 1 instead of an action from the host.
+// The continuation pass re-reads the env action from ro.act_env.  The epilogue writes the path row: reward (its action
+// term on the env action), the done code in path codes, and advances policy_step.  A separate kernel, so that
+// k_tree_step and k_tree_env_step compile exactly as without it.
+template <typename T, int LANES, int ROWS, int CON, int MODE>
+__global__ void __launch_bounds__(kTreeMaxBlock)
+k_tree_rollout_step(const __grid_constant__ TreeModel<T> m, const TreeBatchView<T> v, const __grid_constant__ TreeEnvParams<T> env,
+                    const __grid_constant__ TreeRolloutParams<T> ro, int n_sub, const T* __restrict__ reset_q,
+                    const T* __restrict__ reset_qd, int step_barrier) {
+  typedef EnvScratch<T, ROWS, CON> SC;
+  extern __shared__ __align__(16) unsigned char tree_smem[];
+  const Tile<LANES> tl = Tile<LANES>::make();
+  const int tile_in_block = (int)threadIdx.x / LANES, tiles_per_block = (int)blockDim.x / LANES;
+  const int e_raw = (int)blockIdx.x * tiles_per_block + tile_in_block;
+  const bool active = e_raw < v.n;
+  const int e = active ? e_raw : v.n - 1;
+  int k0 = 0;
+  if (MODE == 2) {
+    k0 = v.resume[e];
+    if (!active || k0 >= n_sub) return;
+  }
+  SC& s = *reinterpret_cast<SC*>(tree_smem + (size_t)tile_in_block * sizeof(SC));
+  const int nq = m.nq, nv = m.nv, nu = m.nu;
+  const T* gq = v.qpos + (size_t)e * nq;
+  const T* gv = v.qvel + (size_t)e * nv;
+  const T* gw = v.warm + (size_t)e * nv;
+  for (int i = tl.lane; i < 7; i += LANES) s.q[i] = gq[i];
+  for (int d = 6 + tl.lane; d < nv; d += LANES) s.q[d + 1] = gq[m.user_dof[d] + 1];
+  for (int d = tl.lane; d < nv; d += LANES) { s.qd[d] = gv[m.user_dof[d]]; s.warm[d] = gw[m.user_dof[d]]; }
+  if (MODE == 2)
+    for (int a = tl.lane; a < nu; a += LANES) s.target[a] = s.ctrl[a] = ro.act_env[(size_t)e * nu + a];
+  if (tl.lane == 0) { s.n_dropped = 0; s.overflow = 0; }
+  tl.sync();
+  if (MODE != 2) {
+    const uint32_t gid = ro.env0 + (uint32_t)e, pstep = (uint32_t)ro.policy_step[e];
+    policy_prologue(tl, m, s, ro.params, ro.lo, ro.hi, ro.normalize,
+                    [&](int a) { return normal_slot<T>(ro.seed, gid, pstep, a); });
+    if (active) {
+      const PolicyStage<T>& ps = policy_stage<T>(s);
+      for (int j = tl.lane; j < kObsDim3d; j += LANES) ro.obs[(size_t)e * kObsDim3d + j] = ps.obs[j];
+      for (int a = tl.lane; a < nu; a += LANES) {
+        const size_t i = (size_t)e * nu + a;
+        ro.act[i] = ps.raw[a];
+        ro.mean[i] = ps.mean[a];
+        ro.act_env[i] = s.target[a];
+      }
+    }
+  }
+  TreeStats st = {0, 0, 0, 0};
+  int k_done = n_sub;
+  bool alive = true;
+  const bool pd = env.mode == kActPd;
+  for (int k = k0; k < n_sub; k++) {
+    if (MODE != 2 && step_barrier > 0 && k % step_barrier == 0) __syncthreads();
+    if (!alive) continue;
+    if (pd) pd_controls(tl, m, s, s.target, env.kp, env.kd);
+    if (!tree_step(tl, m, s, s.ctrl, &st, MODE == 1)) { alive = false; k_done = k; }
+  }
+  if (!active) return;                       // no CTA barrier follows
+  EnvResult r = {0, 0, false};
+  if (alive) {                               // not for an env that is handed on
+    T rew;
+    // the observation env_finish leaves goes to the staging: the next prologue observes the state again
+    r = env_finish(tl, m, s, s.target, kEnvAutoReset, env.max_path_length, reset_q, reset_qd, env.ep_len[e],
+                   policy_stage<T>(s).obs, &rew);
+    if (tl.lane == 0) { ro.rew[e] = rew; env.ep_len[e] = r.len; }
+  }
+  T* oq = v.qpos + (size_t)e * nq;
+  T* ov = v.qvel + (size_t)e * nv;
+  T* ow = v.warm + (size_t)e * nv;
+  for (int i = tl.lane; i < 7; i += LANES) oq[i] = s.q[i];
+  for (int d = 6 + tl.lane; d < nv; d += LANES) oq[m.user_dof[d] + 1] = s.q[d + 1];
+  for (int d = tl.lane; d < nv; d += LANES) { ov[m.user_dof[d]] = s.qd[d]; ow[m.user_dof[d]] = s.warm[d]; }
+  if (tl.lane == 0) {
+    if (MODE != 0) v.resume[e] = k_done;
+    if (alive) {
+      ro.done[e] = (uint8_t)path_done(r.done);
+      ro.policy_step[e] += 1;
       if (n_sub > k0) {
         v.stats[4 * e + 0] = st.nefc; v.stats[4 * e + 1] = st.ncon; v.stats[4 * e + 2] = st.sweeps;
         v.stats[4 * e + 3] += st.dropped;
@@ -280,6 +382,9 @@ struct TreeLaunch {
   static cudaError_t env_step(const TreeModel<T>& m, const TreeBatchView<T>& v, const TreeStepArgs& a, const TreeEnvParams<T>& env,
                               int lanes, cudaStream_t s);
   static cudaError_t observe(const TreeModel<T>& m, const TreeBatchView<T>& v, T* obs, cudaStream_t s);
+  // one policy step of Rollout: a.n_sub, a.reset_q / reset_qd are used
+  static cudaError_t rollout_step(const TreeModel<T>& m, const TreeBatchView<T>& v, const TreeStepArgs& a, const TreeEnvParams<T>& env,
+                                  const TreeRolloutParams<T>& ro, int lanes, cudaStream_t s);
 };
 
 // tiles (envs) per CTA of one kernel instantiation: shared memory is the resource (one Scratch block per env).  Two
@@ -382,6 +487,38 @@ inline cudaError_t launch_tree_env_step(const TreeModel<T>& m, const TreeBatchVi
   return cudaGetLastError();
 }
 
+// the passes of launch_tree_env_step (same knobs, same tiles per CTA: the rollout's per-env block is EnvScratch) on the
+// rollout kernel, for one policy step
+template <typename T, int LANES>
+inline cudaError_t launch_tree_rollout_step(const TreeModel<T>& m, const TreeBatchView<T>& v, const TreeStepArgs& a,
+                                            const TreeEnvParams<T>& env, const TreeRolloutParams<T>& ro, cudaStream_t s) {
+  typedef EnvScratch<T, kFastRows, kFastCon> Fast;
+  typedef EnvScratch<T, kMaxRows, kMaxCon> Full;
+  static const int env_tiles = tree_knob("CASSIE3D_TILES", 0);
+  static const int step_barrier = tree_knob("CASSIE3D_STEP_BARRIER", 1);
+  static const int two_pass = tree_knob("CASSIE3D_TWO_PASS", 1);
+  static const int t_single = tree_tiles(k_tree_rollout_step<T, LANES, kMaxRows, kMaxCon, 0>, sizeof(Full), LANES, env_tiles);
+  static const int t_fast = tree_tiles(k_tree_rollout_step<T, LANES, kFastRows, kFastCon, 1>, sizeof(Fast), LANES, env_tiles);
+  static const int t_cont = tree_tiles(k_tree_rollout_step<T, LANES, kMaxRows, kMaxCon, 2>, sizeof(Full), LANES, 32 / LANES);
+  if (t_single < 0 || t_fast < 0 || t_cont < 0) return cudaErrorInvalidConfiguration;
+  TreeBatchView<T> vv = v;
+  vv.order = nullptr;
+  const T *rq = (const T*)a.reset_q, *rv = (const T*)a.reset_qd;
+  if (!two_pass) {
+    k_tree_rollout_step<T, LANES, kMaxRows, kMaxCon, 0><<<(unsigned)((v.n + t_single - 1) / t_single), t_single * LANES, (size_t)t_single * sizeof(Full), s>>>(
+        m, vv, env, ro, a.n_sub, rq, rv, step_barrier);
+    count_launch();
+    return cudaGetLastError();
+  }
+  k_tree_rollout_step<T, LANES, kFastRows, kFastCon, 1><<<(unsigned)((v.n + t_fast - 1) / t_fast), t_fast * LANES, (size_t)t_fast * sizeof(Fast), s>>>(
+      m, vv, env, ro, a.n_sub, rq, rv, step_barrier);
+  count_launch();
+  k_tree_rollout_step<T, LANES, kMaxRows, kMaxCon, 2><<<(unsigned)((v.n + t_cont - 1) / t_cont), t_cont * LANES, (size_t)t_cont * sizeof(Full), s>>>(
+      m, vv, env, ro, a.n_sub, rq, rv, 0);
+  count_launch();
+  return cudaGetLastError();
+}
+
 #define CASSIE_TREE_INSTANTIATE(T)                                                                                         \
   template <>                                                                                                              \
   cudaError_t TreeLaunch<T>::step(const TreeModel<T>& dm, const TreeBatchView<T>& v, const TreeStepArgs& a, int lanes,     \
@@ -411,6 +548,15 @@ inline cudaError_t launch_tree_env_step(const TreeModel<T>& m, const TreeBatchVi
     k_tree_observe<T><<<(v.n + kObsTiles - 1) / kObsTiles, kObsLanes * kObsTiles, 0, s>>>(dm, v, obs);                     \
     count_launch();                                                                                                        \
     return cudaGetLastError();                                                                                             \
+  }                                                                                                                        \
+  template <>                                                                                                              \
+  cudaError_t TreeLaunch<T>::rollout_step(const TreeModel<T>& dm, const TreeBatchView<T>& v, const TreeStepArgs& a,        \
+                                          const TreeEnvParams<T>& env, const TreeRolloutParams<T>& ro, int lanes,          \
+                                          cudaStream_t s) {                                                                \
+    if (lanes == 8) return launch_tree_rollout_step<T, 8>(dm, v, a, env, ro, s);                                           \
+    if (lanes == 16) return launch_tree_rollout_step<T, 16>(dm, v, a, env, ro, s);                                         \
+    if (lanes == 32) return launch_tree_rollout_step<T, 32>(dm, v, a, env, ro, s);                                         \
+    return cudaErrorInvalidValue;                                                                                          \
   }
 
 }  // namespace tree

@@ -1,6 +1,7 @@
 """Rollout collection for the reference's TRPO launcher (rllab/envs/trpo_cassie.py:13-55), batched:
 GaussianMLPPolicy(hidden_sizes=(32, 32)) + normalize(Cassie2dEnv) + rollout(max_path_length), fused in
-one CUDA kernel per T policy steps (csrc/rollout_kernels.cuh).  Paths come back in rllab's dict layout
+one CUDA kernel per T policy steps (csrc/rollout_kernels.cuh); RolloutCollector3d does the same on the 3-D stand env
+(csrc/tree_rollout.cuh, one launch pass per policy step).  Paths come back in rllab's dict layout
 (SURVEY App. E): observations[T,odim], actions[T,adim] (raw policy outputs), rewards[T],
 agent_infos{mean, log_std}, env_infos{}.  The TRPO update itself is rllab's and out of scope.
 """
@@ -57,7 +58,52 @@ class GaussianMLPPolicy:
         return self.unpack()[6]
 
 
-class RolloutCollector:
+class _PathSampler:
+    """Host side shared by the planar and the 3-D collector: the LinearFeatureBaseline solve on the device-accumulated
+    normal equations and the split of the [T, N, .] buffers into rllab paths.  Needs batch, obs_dim, act_dim, _T."""
+
+    def _buffers(self, T):
+        if T != self._T:
+            b, n = self.batch, self.batch.n
+            mk = lambda *s, dt=None: torch.empty(s, dtype=dt or b.dtype, device=b.device)
+            self.obs, self.act, self.mean = mk(T, n, self.obs_dim), mk(T, n, self.act_dim), mk(T, n, self.act_dim)
+            self.rew, self.done = mk(T, n), mk(T, n, dt=torch.uint8)
+            self._T = T
+
+    def _solve_baseline(self, mom, D, reg_coeff):
+        m = mom.cpu().numpy()
+        FtF = np.zeros((D, D)); iu = np.triu_indices(D)
+        FtF[iu] = m[:D * (D + 1) // 2]; FtF = FtF + FtF.T - np.diag(np.diag(FtF))
+        Fty = m[D * (D + 1) // 2:]
+        self.baseline_moments = (FtF, Fty)
+        coeffs = None
+        for _ in range(5):                           # rllab retries with a 10x larger regulariser on NaNs
+            coeffs = np.linalg.lstsq(FtF + reg_coeff * np.eye(D), Fty, rcond=None)[0]
+            if not np.any(np.isnan(coeffs)):
+                break
+            reg_coeff *= 10
+        b = self.batch
+        self.baseline_coeffs = torch.tensor(coeffs, dtype=b.dtype, device=b.device)
+        return self.baseline_coeffs
+
+    def paths(self, policy, envs=None):
+        """Split the last collect() into rllab path dicts (one per finished or truncated episode)."""
+        obs, act, mean, rew, done = (x.cpu().numpy() for x in (self.obs, self.act, self.mean, self.rew, self.done))
+        log_std = policy.log_std.cpu().numpy()
+        out = []
+        for e in (range(obs.shape[1]) if envs is None else envs):
+            start = 0
+            ends = list(np.nonzero(done[:, e])[0]) + ([obs.shape[0] - 1] if done[-1, e] == 0 else [])
+            for k in ends:
+                sl = slice(start, k + 1)
+                out.append(dict(observations=obs[sl, e], actions=act[sl, e], rewards=rew[sl, e],
+                                agent_infos=dict(mean=mean[sl, e], log_std=np.tile(log_std, (k + 1 - start, 1))),
+                                env_infos={}, env=e, start=start, terminated=bool(done[k, e] == 1)))
+                start = k + 1
+        return out
+
+
+class RolloutCollector(_PathSampler):
     """Owns the env batch and the [T, N, .] path buffers; `collect(T)` launches one kernel."""
 
     def __init__(self, n_envs, device=0, task="stand", control_mode="OSC", precision=32, max_path_length=1000,
@@ -80,14 +126,6 @@ class RolloutCollector:
         with torch.cuda.device(b.device):
             _lib.check(b.L.Cassie2dBatchEnvReset(b.h, self.task, self.flags, None, _stream_ptr()), "EnvReset")
         self._T = 0
-
-    def _buffers(self, T):
-        if T != self._T:
-            b, n = self.batch, self.batch.n
-            mk = lambda *s, dt=None: torch.empty(s, dtype=dt or b.dtype, device=b.device)
-            self.obs, self.act, self.mean = mk(T, n, self.obs_dim), mk(T, n, self.act_dim), mk(T, n, self.act_dim)
-            self.rew, self.done = mk(T, n), mk(T, n, dt=torch.uint8)
-            self._T = T
 
     def collect(self, policy, T):
         self._buffers(T)
@@ -130,19 +168,7 @@ class RolloutCollector:
             _lib.check(b.L.Cassie2dBatchBaselineMoments(b.h, self.task, self.obs.data_ptr(), returns.data_ptr(), self.done.data_ptr(),
                                                         self._path_start.data_ptr(), int(T), self._pidx.data_ptr(), mom.data_ptr(),
                                                         _stream_ptr()), "BaselineMoments")
-        m = mom.cpu().numpy()
-        FtF = np.zeros((D, D)); iu = np.triu_indices(D)
-        FtF[iu] = m[:D * (D + 1) // 2]; FtF = FtF + FtF.T - np.diag(np.diag(FtF))
-        Fty = m[D * (D + 1) // 2:]
-        self.baseline_moments = (FtF, Fty)
-        coeffs = None
-        for _ in range(5):                           # rllab retries with a 10x larger regulariser on NaNs
-            coeffs = np.linalg.lstsq(FtF + reg_coeff * np.eye(D), Fty, rcond=None)[0]
-            if not np.any(np.isnan(coeffs)):
-                break
-            reg_coeff *= 10
-        self.baseline_coeffs = torch.tensor(coeffs, dtype=b.dtype, device=b.device)
-        return self.baseline_coeffs
+        return self._solve_baseline(mom, D, reg_coeff)
 
     def advantages(self, gamma=0.99, gae_lambda=1.0, coeffs=None):
         """GAE advantages and baseline values [T, N] of the last collect() (after fit_baseline)."""
@@ -155,21 +181,93 @@ class RolloutCollector:
                                                    adv.data_ptr(), val.data_ptr(), _stream_ptr()), "Advantages")
         return adv, val
 
-    def paths(self, policy, envs=None):
-        """Split the last collect() into rllab path dicts (one per finished or truncated episode)."""
-        obs, act, mean, rew, done = (x.cpu().numpy() for x in (self.obs, self.act, self.mean, self.rew, self.done))
-        log_std = policy.log_std.cpu().numpy()
-        out = []
-        for e in (range(obs.shape[1]) if envs is None else envs):
-            start = 0
-            ends = list(np.nonzero(done[:, e])[0]) + ([obs.shape[0] - 1] if done[-1, e] == 0 else [])
-            for k in ends:
-                sl = slice(start, k + 1)
-                out.append(dict(observations=obs[sl, e], actions=act[sl, e], rewards=rew[sl, e],
-                                agent_infos=dict(mean=mean[sl, e], log_std=np.tile(log_std, (k + 1 - start, 1))),
-                                env_infos={}, env=e, start=start, terminated=bool(done[k, e] == 1)))
-                start = k + 1
-        return out
+    def close(self):
+        self.batch.close()
+
+
+class RolloutCollector3d(_PathSampler):
+    """The planar collector's interface on the 3-D stand env (include/cassie3d.h, Cassie3dBatchRollout):
+    GaussianMLPPolicy(45, 10) + normalize(Cassie3dBatchEnv) + rollout(max_path_length).  `collect(policy, T)` enqueues
+    one launch pass per policy step (the policy forward, the noise and the action map are fused into the env step) and
+    returns the same dict as RolloutCollector.collect; dones are path codes: 1 terminated (fell or diverged), 2 cut at
+    max_path_length.  Episodes continue across collect() calls."""
+
+    def __init__(self, n_envs, device=0, control_mode="PD", precision=32, max_path_length=1000, n_substeps=10,
+                 normalize=True, seed=1, first_global_env=0, lanes=None):
+        from .envs3d import MODE3D_BY_NAME, Cassie3dBatch
+        if control_mode not in MODE3D_BY_NAME:
+            raise ValueError("control_mode must be 'PD' or 'Torque'")
+        self.batch = Cassie3dBatch(n_envs, device, precision, lanes=lanes)
+        self.control_mode, self.mode = control_mode, MODE3D_BY_NAME[control_mode]
+        self.obs_dim, self.act_dim = _lib.OBS_DIM_3D, self.batch.nu
+        self.max_path_length, self.n_substeps, self.normalize = int(max_path_length), int(n_substeps), normalize
+        self.seed, self.env0 = seed, first_global_env
+        b = self.batch
+        with torch.cuda.device(b.device):
+            self._check(b.L.Cassie3dBatchEnvReset(b.h, None, None, _stream_ptr()), "EnvReset")
+        self._T = 0
+        self._path_start = torch.empty(b.n, dtype=torch.int32, device=b.device)
+
+    @staticmethod
+    def _check(rc, what):
+        from .envs3d import _check
+        _check(rc, what)
+
+    @property
+    def action_space(self):
+        """(lb, ub) of the action map and clip, as the library takes them from the model"""
+        lo, hi = np.zeros(self.act_dim), np.zeros(self.act_dim)
+        dp = _lib.ct.POINTER(_lib.ct.c_double)
+        self._check(self.batch.L.Cassie3dBatchActionBox(self.batch.h, self.mode, lo.ctypes.data_as(dp), hi.ctypes.data_as(dp)), "ActionBox")
+        return lo, hi
+
+    def collect(self, policy, T):
+        self._buffers(T)
+        b = self.batch
+        p = policy.flat.to(dtype=b.dtype, device=b.device).contiguous()
+        with torch.cuda.device(b.device):
+            # where each env's current path stands: the in-path index of this batch's first samples (baseline features)
+            self._check(b.L.Cassie3dBatchGetEpisodeLengths(b.h, self._path_start.data_ptr(), _stream_ptr()), "GetEpisodeLengths")
+            self._check(b.L.Cassie3dBatchRollout(
+                b.h, self.mode, p.data_ptr(), p.numel(), int(T), self.n_substeps, self.max_path_length, int(self.normalize),
+                self.seed, self.env0, self.obs.data_ptr(), self.act.data_ptr(), self.mean.data_ptr(), self.rew.data_ptr(),
+                self.done.data_ptr(), _stream_ptr()), "Rollout")
+        return dict(observations=self.obs, actions=self.act, means=self.mean, rewards=self.rew, dones=self.done)
+
+    def discounted_returns(self, gamma=0.99, tail=None):
+        """returns[T, N] of the last collect(), on device; unfinished paths bootstrapped with `tail` (real [N]) or 0"""
+        b = self.batch
+        ret = torch.empty_like(self.rew)
+        with torch.cuda.device(b.device):
+            self._check(b.L.Cassie3dBatchDiscountedReturns(b.h, self.rew.data_ptr(), self.done.data_ptr(),
+                                                           tail.data_ptr() if tail is not None else None, float(gamma),
+                                                           int(self._T), ret.data_ptr(), _stream_ptr()), "DiscountedReturns")
+        return ret
+
+    def fit_baseline(self, returns, reg_coeff=1e-5):
+        """LinearFeatureBaseline.fit: normal equations (D = 94) accumulated on device, the solve on the host"""
+        b = self.batch
+        D = 2 * self.obs_dim + 4
+        T = self._T
+        if getattr(self, "_pidx", None) is None or self._pidx.shape[0] != T:
+            self._pidx = torch.empty((T, b.n), dtype=torch.int32, device=b.device)
+        mom = torch.empty(D * (D + 1) // 2 + D, dtype=torch.float64, device=b.device)
+        with torch.cuda.device(b.device):
+            self._check(b.L.Cassie3dBatchBaselineMoments(b.h, self.obs.data_ptr(), returns.data_ptr(), self.done.data_ptr(),
+                                                         self._path_start.data_ptr(), int(T), self._pidx.data_ptr(), mom.data_ptr(),
+                                                         _stream_ptr()), "BaselineMoments")
+        return self._solve_baseline(mom, D, reg_coeff)
+
+    def advantages(self, gamma=0.99, gae_lambda=1.0, coeffs=None):
+        """GAE advantages and baseline values [T, N] of the last collect() (after fit_baseline)."""
+        b = self.batch
+        c = self.baseline_coeffs if coeffs is None else coeffs
+        adv = torch.empty_like(self.rew); val = torch.empty_like(self.rew)
+        with torch.cuda.device(b.device):
+            self._check(b.L.Cassie3dBatchAdvantages(b.h, self.obs.data_ptr(), self.rew.data_ptr(), self.done.data_ptr(),
+                                                    self._pidx.data_ptr(), c.data_ptr(), float(gamma), float(gae_lambda),
+                                                    int(self._T), adv.data_ptr(), val.data_ptr(), _stream_ptr()), "Advantages")
+        return adv, val
 
     def close(self):
         self.batch.close()

@@ -95,6 +95,51 @@ int Cassie3dBatchObserve(Cassie3dBatch* h, void* obs, void* stream);
 /* int32 [n]: EnvStep calls since each env's last reset */
 int Cassie3dBatchGetEpisodeLengths(Cassie3dBatch* h, int32_t* ep_len, void* stream);
 
+/* ---- rollout collection on the stand-task env (the planar Cassie2dBatchRollout's counterpart): rllab's BatchSampler
+ * with GaussianMLPPolicy(hidden_sizes=(32, 32)) and normalize(env), n_policy_steps policy steps of every env, enqueued
+ * on `stream` without a host synchronisation (one or two launches per policy step).
+ *
+ * Per env and policy step k: obs[k] = the observation of the current state; mean[k] = tanh MLP 45 -> 32 -> 32 -> 10 with
+ * a linear head, params_dev = rllab's flat vector W1 b1 W2 b2 W3 b3 log_std (real, W stored [in][out],
+ * CASSIE3D_POLICY_PARAMS entries); action[k] = mean + exp(log_std) * eps, the raw policy output rllab stores; the env
+ * action = lb + (action + 1) / 2 (ub - lb) clipped to [lb, ub] with normalize != 0, else action clipped; then
+ * n_substeps >= 1 simulator steps and the EnvStep epilogue with auto-reset: reward[k] (its action term on the env
+ * action), done[k] in path codes 1 = terminated (fell or diverged; a diverged env's reward is 0), 2 = cut because the
+ * episode length reached max_path_length > 0, else 0.  Episodes continue across calls; the episode lengths are
+ * EnvStep's (GetEpisodeLengths).
+ *
+ * Buffers (device): obs real [T][n][CASSIE3D_OBS_DIM], action / mean real [T][n][nu], reward real [T][n], done uint8
+ * [T][n], T = n_policy_steps.
+ * Action box [lb, ub] (Cassie3dBatchActionBox), from the model: CASSIE3D_MODE_TORQUE the motors' ctrlrange,
+ * CASSIE3D_MODE_PD the range of each motor's joint.
+ * Noise: eps of action a = Box-Muller on Philox4x32-10 with key = seed (low word first) and counter {first_global_env +
+ * e, step, a / 4, 0}, step = the env's rollout policy-step counter (0 at Create, advanced by Rollout only, never reset):
+ * actions 0..7 are the two pairs of blocks 0 and 1 as in the planar rollout, actions 8 and 9 the first pair of block 2.
+ * A batch holding global envs [first_global_env, first_global_env + n) therefore draws what one large batch would. */
+enum { CASSIE3D_POLICY_PARAMS = 2868 };
+int Cassie3dBatchRollout(Cassie3dBatch* h, int mode, const void* params_dev, int n_params, int n_policy_steps,
+                         int n_substeps, int max_path_length, int normalize, unsigned long long seed,
+                         unsigned int first_global_env, void* obs_dev, void* action_dev, void* mean_dev,
+                         void* reward_dev, uint8_t* done_dev, void* stream);
+/* host doubles [nu]: the action box Rollout maps into and clips to in `mode` */
+int Cassie3dBatchActionBox(Cassie3dBatch* h, int mode, double* lo, double* hi);
+/* sampler side of rllab's process_samples on Rollout's [T][n] buffers, as the planar calls of the same names:
+ * returns[k] = reward[k] + gamma returns[k + 1] within a path, the last unfinished path bootstrapped with tail_dev
+ * (real [n], NULL = 0) */
+int Cassie3dBatchDiscountedReturns(Cassie3dBatch* h, const void* reward_dev, const uint8_t* done_dev, const void* tail_dev,
+                                   double gamma, int n_policy_steps, void* returns_dev, void* stream);
+/* LinearFeatureBaseline normal equations: features [clip(o, -10, 10), clip(o)^2, al, al^2, al^3, 1], al = step in path
+ * / 100 (D = 94); path_start_dev (int32 [n], may be NULL = 0) = the in-path index of each env's first sample,
+ * path_index_dev (int32 [T][n]) receives every sample's; moments_dev (double, D (D + 1) / 2 + D) = the packed upper
+ * triangle of F'F row by row, then F'y */
+int Cassie3dBatchBaselineMoments(Cassie3dBatch* h, const void* obs_dev, const void* returns_dev, const uint8_t* done_dev,
+                                 const int32_t* path_start_dev, int n_policy_steps, int32_t* path_index_dev,
+                                 double* moments_dev, void* stream);
+/* baseline values (values_dev may be NULL) and GAE advantages [T][n] with the coefficients coeffs_dev (real [D]) */
+int Cassie3dBatchAdvantages(Cassie3dBatch* h, const void* obs_dev, const void* reward_dev, const uint8_t* done_dev,
+                            const int32_t* path_index_dev, const void* coeffs_dev, double gamma, double gae_lambda,
+                            int n_policy_steps, void* advantages_dev, void* values_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -3,7 +3,13 @@ sampler-side pre-processing (returns, LinearFeatureBaseline fit, GAE advantages)
 bench (bench.py); prints one JSON line for profiles/.
 
   python tools/bench_rollout.py [--envs N] [--T T] [--mode PD|OSC|TORQUE]
+  python tools/bench_rollout.py --model 3d [--envs N] [--T T] [--mode PD|TORQUE]      # the 3-D stand env
   python -m torch.distributed.run --nproc-per-node G ... tools/bench_rollout.py     # N envs PER GPU, one rank per GPU
+
+--model 3d (RolloutCollector3d, default 8192 envs per GPU, T = 20, PD) also times, in the same process and alternated
+twice, the loop a user would otherwise write on Cassie3dBatchEnv (PyTorch policy forward, randn, affine map, clamp,
+EnvStep) and EnvStep alone on pre-generated actions (an upper bound for the fused collect), and reports the rollout and
+env kernels' launch resources read from a torch.profiler trace, with the card's name and power limit.
 
 Multi-GPU (SURVEY 8e): envs are sharded by global env id (Philox streams and phases do not depend on G), there is no
 collective inside a rollout; after it, NCCL all-reduces the rollout statistics (cassierl_b200.parallel.RolloutStats) and
@@ -13,7 +19,9 @@ rollout.  Times are CUDA-event times, max over ranks.
 import argparse
 import json
 import os
+import subprocess
 import sys
+import tempfile
 import time
 
 import torch
@@ -21,15 +29,20 @@ import torch.distributed as dist
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from cassierl_b200 import parallel  # noqa: E402
-from cassierl_b200.rollout import GaussianMLPPolicy, RolloutCollector  # noqa: E402
+from cassierl_b200.rollout import GaussianMLPPolicy, RolloutCollector, RolloutCollector3d  # noqa: E402
 
 p = argparse.ArgumentParser()
-p.add_argument("--envs", type=int, default=16384, help="envs per GPU")
+p.add_argument("--model", default="2d", choices=["2d", "3d"], help="planar (cassie2d) or 3-D (cassie3d stand env)")
+p.add_argument("--envs", type=int, default=None, help="envs per GPU (default 16384 planar, 8192 3-D)")
 p.add_argument("--T", type=int, default=20, help="policy steps per collect() (10 sim steps each)")
 p.add_argument("--reps", type=int, default=5)
 p.add_argument("--mode", default="PD", choices=["PD", "OSC", "TORQUE"])
 p.add_argument("--task", default="stand", choices=["stand", "imitate"])
 a = p.parse_args()
+if a.envs is None:
+    a.envs = 8192 if a.model == "3d" else 16384
+if a.model == "3d" and a.mode == "OSC":
+    p.error("the 3-D env offers PD and TORQUE")
 
 world = int(os.environ.get("WORLD_SIZE", "1")); rank = int(os.environ.get("RANK", "0")); local = int(os.environ.get("LOCAL_RANK", "0"))
 torch.cuda.set_device(local)
@@ -38,7 +51,11 @@ if world > 1:
     dist.init_process_group("nccl", device_id=dev)
 n_total = a.envs * world
 
-col = RolloutCollector(a.envs, device=local, task=a.task, control_mode=a.mode, max_path_length=1000, first_global_env=rank * a.envs)
+if a.model == "3d":
+    col = RolloutCollector3d(a.envs, device=local, control_mode={"PD": "PD", "TORQUE": "Torque"}[a.mode], max_path_length=1000,
+                             first_global_env=rank * a.envs)
+else:
+    col = RolloutCollector(a.envs, device=local, task=a.task, control_mode=a.mode, max_path_length=1000, first_global_env=rank * a.envs)
 pol = GaussianMLPPolicy(col.obs_dim, col.act_dim, device=dev)
 if world > 1:
     dist.broadcast(pol.flat, src=0)            # the learner's parameters (8.5 kB), once per iteration
@@ -67,7 +84,93 @@ def timed(fn, reps):
     return maxr(sorted(ms)[len(ms) // 2])
 
 
+def card():
+    """name, power limit and max SM clock of this rank's GPU (nvidia-smi query; read in the measuring process)"""
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", str(torch.cuda.current_device()), "--query-gpu=name,power.limit,clocks.max.sm",
+                            "--format=csv,noheader"], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        q = ""
+    return {"name": torch.cuda.get_device_name(dev), "nvidia_smi": q or "unavailable"}
+
+
+def kernel_resources(fns, names):
+    """launch resources of the kernels whose name contains one of `names`, from a torch.profiler trace of fns (the
+    trace goes to a temporary directory)"""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for fn in fns:
+            fn()
+        torch.cuda.synchronize()
+    with tempfile.TemporaryDirectory() as td:
+        path = os.path.join(td, "trace.json")
+        prof.export_chrome_trace(path)
+        with open(path) as f:
+            events = json.load(f)["traceEvents"]
+    out = {}
+    for ev in events:
+        if ev.get("cat") != "kernel":
+            continue
+        for nm in names:
+            if nm + "<" in ev["name"] or ev["name"].startswith(nm):
+                ar = ev.get("args", {})
+                key = ev["name"].split("(")[0].replace("void ", "").replace("cassie::tree::", "")
+                out.setdefault(key, {k: ar.get(k) for k in ("registers per thread", "shared memory", "block", "grid",
+                                                             "blocks per SM", "warps per SM", "est. achieved occupancy %")})
+    return out
+
+
+def compare_3d():
+    """(a) the fused collect, (b) the unfused loop on Cassie3dBatchEnv, (c) EnvStep alone on pre-generated actions;
+    same envs, policy and T, alternated twice, CUDA-event times (median of --reps each)"""
+    from cassierl_b200.envs3d import Cassie3dBatchEnv
+    env = Cassie3dBatchEnv(a.envs, device=local, control_mode=col.control_mode, auto_reset=True, max_path_length=1000)
+    env.reset()
+    n, T = a.envs, a.T
+    lo, hi = (torch.tensor(x, dtype=env.batch.dtype, device=dev) for x in col.action_space)
+    W1, b1, W2, b2, W3, b3, log_std = pol.unpack()
+    std = log_std.exp()
+    mk = lambda *sh, dt=env.batch.dtype: torch.empty(sh, dtype=dt, device=dev)
+    bo, ba, bm, br, bd = mk(T, n, 45), mk(T, n, 10), mk(T, n, 10), mk(T, n), mk(T, n, dt=torch.uint8)
+    state = {"obs": env.observe().clone()}
+
+    def unfused():
+        o = state["obs"]
+        for k in range(T):
+            h = torch.tanh(o @ W1 + b1)
+            h = torch.tanh(h @ W2 + b2)
+            mean = h @ W3 + b3
+            act = mean + std * torch.randn_like(mean)
+            x = (lo + (act + 1.0) * 0.5 * (hi - lo)).clamp(lo, hi)
+            bo[k].copy_(o); ba[k].copy_(act); bm[k].copy_(mean)
+            o, r, d = env.step(x)
+            br[k].copy_(r); bd[k].copy_(d)
+        state["obs"] = o
+
+    pre = (lo + (torch.rand(T, n, 10, device=dev, dtype=env.batch.dtype)) * (hi - lo)).contiguous()
+
+    def env_only():
+        for k in range(T):
+            env.step(pre[k])
+
+    unfused(); env_only(); torch.cuda.synchronize()                      # warm-up of every shape
+    runs = {"fused_collect": [], "unfused_loop": [], "env_step_only": []}
+    for _ in range(2):
+        runs["fused_collect"].append(timed(lambda: col.collect(pol, T), a.reps))
+        runs["unfused_loop"].append(timed(unfused, a.reps))
+        runs["env_step_only"].append(timed(env_only, a.reps))
+    res = kernel_resources([lambda: col.collect(pol, 2), lambda: env.step(pre[0])], ["k_tree_rollout_step", "k_tree_env_step"])
+    best = {k: min(v) for k, v in runs.items()}
+    env.terminate()
+    return {"ms_per_collect": runs,
+            "env_steps_per_s": {k: [n * T * 10 / (x * 1e-3) for x in v] for k, v in runs.items()},
+            "fused_vs_env_step_only": best["fused_collect"] / best["env_step_only"] - 1.0,
+            "fused_vs_unfused": best["fused_collect"] / best["unfused_loop"] - 1.0,
+            "kernels": res, "card": card()}
+
+
 ms_collect = timed(lambda: col.collect(pol, a.T), a.reps)
+cmp3d = compare_3d() if a.model == "3d" else None
 t0 = time.perf_counter()
 for _ in range(a.reps):
     ret = col.discounted_returns(); col.fit_baseline(ret); col.advantages()
@@ -112,6 +215,22 @@ if world > 1:
               "collect_plus_gather_serial_ms": ms_collect + ms_gather, "collect_with_overlapped_gather_ms": ms_overlap}
 
 d = col.done
+if a.model == "3d":
+    st = col.batch.stats().double()   # [n, 4]: constraint rows, contacts, PGS sweeps, contacts dropped
+    if rank == 0:
+        print(json.dumps({
+            "workload": "rollout: GaussianMLPPolicy(45->32->32->10) + %s action space + cassie3d stand env, %d envs per GPU x %d GPUs x %d policy steps x 10 sim steps"
+                        % (col.control_mode, a.envs, world, a.T),
+            "n_gpus": world, "collect_ms": ms_collect, "env_steps_per_s": n_total * a.T * 10 / (ms_collect * 1e-3),
+            "policy_steps_per_s": n_total * a.T / (ms_collect * 1e-3),
+            "env_steps_per_s_with_overlapped_gather": (n_total * a.T * 10 / (gather["collect_with_overlapped_gather_ms"] * 1e-3)) if world > 1 else None,
+            "returns_baseline_advantages_ms": ms_post, "episodes_finished": int((d != 0).sum().item()),
+            "rollout_stats_all_ranks": red, "gather": gather, "compare_rank0": cmp3d,
+            "last_step_rows_mean": float(st[:, 0].mean().item()), "last_step_rows_max": int(st[:, 0].max().item())}), flush=True)
+    if world > 1:
+        dist.barrier()
+        dist.destroy_process_group()
+    sys.exit(0)
 st = col.batch.stats().double()   # [n, 4]: rows, PGS sweeps, QP iterations, QP status of the last sim step
 qp = {"iters_mean": float(st[:, 2].mean().item()), "iters_max": int(st[:, 2].max().item()),
       "iters_p99": float(torch.quantile(st[:, 2], 0.99).item()), "not_optimal": int((st[:, 3] != 0).sum().item()),
