@@ -139,9 +139,9 @@ int env_step(Cassie3dBatch* h, int mode, const void* action, int n_sub, int max_
 }
 
 template <typename T>
-int rollout(Cassie3dBatch* h, int mode, const void* params, int T_steps, int n_sub, int max_path_length, int normalize,
-            unsigned long long seed, unsigned int env0, void* obs, void* act, void* mean, void* reward, uint8_t* done,
-            cudaStream_t s) {
+int rollout(Cassie3dBatch* h, int mode, const PolicyShape3d& shape, const void* params, int T_steps, int n_sub,
+            int max_path_length, int normalize, unsigned long long seed, unsigned int env0, void* obs, void* act, void* mean,
+            void* reward, uint8_t* done, cudaStream_t s) {
   const size_t n = (size_t)h->n, nu = (size_t)h->model.nu;
   TreeStepArgs a;
   a.action = nullptr; a.n_sub = n_sub; a.z_done = 0; a.auto_reset = 1; a.done = nullptr;
@@ -157,7 +157,7 @@ int rollout(Cassie3dBatch* h, int mode, const void* params, int T_steps, int n_s
   double lo[kMaxAct] = {0}, hi[kMaxAct] = {0};
   action_box(h->model, mode, lo, hi);
   for (int i = 0; i < kMaxAct; i++) { ro.lo[i] = (T)lo[i]; ro.hi[i] = (T)hi[i]; }
-  ro.params = (const T*)params; ro.normalize = normalize; ro.seed = seed; ro.env0 = env0;
+  ro.params = (const T*)params; ro.shape = shape; ro.normalize = normalize; ro.seed = seed; ro.env0 = env0;
   ro.policy_step = h->policy_step; ro.act_env = (T*)h->d_act_env;
   for (int k = 0; k < T_steps; k++) {   // one launch pass per policy step, no host synchronisation in between
     ro.obs = (T*)obs + (size_t)k * n * kObsDim3d;
@@ -190,6 +190,8 @@ static_assert((int)CASSIE3D_MODE_TORQUE == (int)kActTorque && (int)CASSIE3D_MODE
 static_assert((int)CASSIE3D_AUTO_RESET == (int)kEnvAutoReset && (int)CASSIE3D_TERMINAL_OBS == (int)kEnvTerminalObs, "env flags");
 static_assert((int)CASSIE3D_OBS_DIM == kObsDim3d, "observation size");
 static_assert((int)CASSIE3D_POLICY_PARAMS == kPolicyParams3d, "policy parameter count");
+static_assert((int)CASSIE3D_POLICY_MAX_LAYERS == kPolicyMaxLayers3d && (int)CASSIE3D_POLICY_MAX_WIDTH == kPolicyMaxWidth3d,
+              "policy shape limits");
 static_assert(kMaxFeat3d == 2 * kObsDim3d + 4, "baseline features of the 3-D observation");
 
 #define DISPATCH3(h, expr32, expr64) ((h)->precision == 64 ? (expr64) : (expr32))
@@ -422,24 +424,44 @@ int Cassie3dBatchObserve(Cassie3dBatch* h, void* obs, void* stream) {
   return DISPATCH3(h, observe<float>(h, obs, s), observe<double>(h, obs, s));
 }
 
-int Cassie3dBatchRollout(Cassie3dBatch* h, int mode, const void* params_dev, int n_params, int n_policy_steps,
-                         int n_substeps, int max_path_length, int normalize, unsigned long long seed,
-                         unsigned int first_global_env, void* obs_dev, void* action_dev, void* mean_dev,
-                         void* reward_dev, uint8_t* done_dev, void* stream) {
-  if (!h || !params_dev || !obs_dev || !action_dev || !mean_dev || !reward_dev || !done_dev) return fail3("null argument");
+int Cassie3dBatchRolloutMlp(Cassie3dBatch* h, int mode, int n_hidden, const int32_t* hidden_sizes, const void* params_dev,
+                            int n_params, int n_policy_steps, int n_substeps, int max_path_length, int normalize,
+                            unsigned long long seed, unsigned int first_global_env, void* obs_dev, void* action_dev,
+                            void* mean_dev, void* reward_dev, uint8_t* done_dev, void* stream) {
+  if (!h || !hidden_sizes || !params_dev || !obs_dev || !action_dev || !mean_dev || !reward_dev || !done_dev)
+    return fail3("null argument");
   if (mode != CASSIE3D_MODE_TORQUE && mode != CASSIE3D_MODE_PD) return fail3("mode must be CASSIE3D_MODE_TORQUE or CASSIE3D_MODE_PD");
   if (n_policy_steps < 0) return fail3("n_policy_steps must not be negative");
   if (n_substeps < 1) return fail3("n_substeps must be at least 1");
   if (max_path_length <= 0) return fail3("max_path_length must be positive");
-  if (n_params != kPolicyParams3d)
-    return fail3("policy parameter vector has " + std::to_string(n_params) + " entries, expected " + std::to_string(kPolicyParams3d));
+  if (n_hidden < 1 || n_hidden > kPolicyMaxLayers3d)
+    return fail3("n_hidden is " + std::to_string(n_hidden) + ", the policy takes 1 to " + std::to_string(kPolicyMaxLayers3d) + " hidden layers");
+  PolicyShape3d shape = {n_hidden, {0, 0, 0, 0}};
+  for (int l = 0; l < n_hidden; l++) {
+    if (hidden_sizes[l] < 1 || hidden_sizes[l] > kPolicyMaxWidth3d)
+      return fail3("hidden_sizes[" + std::to_string(l) + "] is " + std::to_string(hidden_sizes[l]) + ", a hidden layer has 1 to " +
+                   std::to_string(kPolicyMaxWidth3d) + " units");
+    shape.width[l] = hidden_sizes[l];
+  }
+  const int want = policy_params3d(shape);
+  if (n_params != want)
+    return fail3("policy parameter vector has " + std::to_string(n_params) + " entries, expected " + std::to_string(want));
   if (h->model.nu != kPolicyAct3d) return fail3("the policy has " + std::to_string(kPolicyAct3d) + " actions, the model " + std::to_string(h->model.nu) + " motors");
   DeviceGuard g(h->device);
   cudaStream_t s = (cudaStream_t)stream;
-  return DISPATCH3(h, rollout<float>(h, mode, params_dev, n_policy_steps, n_substeps, max_path_length, normalize, seed,
+  return DISPATCH3(h, rollout<float>(h, mode, shape, params_dev, n_policy_steps, n_substeps, max_path_length, normalize, seed,
                                      first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s),
-                   rollout<double>(h, mode, params_dev, n_policy_steps, n_substeps, max_path_length, normalize, seed,
+                   rollout<double>(h, mode, shape, params_dev, n_policy_steps, n_substeps, max_path_length, normalize, seed,
                                    first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s));
+}
+
+int Cassie3dBatchRollout(Cassie3dBatch* h, int mode, const void* params_dev, int n_params, int n_policy_steps,
+                         int n_substeps, int max_path_length, int normalize, unsigned long long seed,
+                         unsigned int first_global_env, void* obs_dev, void* action_dev, void* mean_dev,
+                         void* reward_dev, uint8_t* done_dev, void* stream) {
+  static const int32_t kDefault[2] = {kPolicyHidden3d, kPolicyHidden3d};
+  return Cassie3dBatchRolloutMlp(h, mode, 2, kDefault, params_dev, n_params, n_policy_steps, n_substeps, max_path_length,
+                                 normalize, seed, first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, stream);
 }
 
 int Cassie3dBatchActionBox(Cassie3dBatch* h, int mode, double* lo, double* hi) {

@@ -210,7 +210,8 @@ k_tree_env_step(const __grid_constant__ TreeModel<T> m, const TreeBatchView<T> v
 template <typename T>
 struct TreeRolloutParams {
   T lo[kMaxAct], hi[kMaxAct];   // action box: ctrlrange (torque mode) or the motors' joint ranges (PD mode)
-  const T* params;              // [kPolicyParams3d] GaussianMLPPolicy.flat
+  const T* params;              // [policy_params3d(shape)] GaussianMLPPolicy.flat
+  PolicyShape3d shape;          // hidden_sizes
   int normalize;                // NormalizedEnv's affine map before the clip
   uint64_t seed;
   uint32_t env0;                // global id of this batch's env 0
@@ -260,7 +261,7 @@ k_tree_rollout_step(const __grid_constant__ TreeModel<T> m, const TreeBatchView<
   if (MODE != 2) {
     const uint32_t gid = ro.env0 + (uint32_t)e, pstep = (uint32_t)ro.policy_step[e];
     policy_prologue(tl, m, s, ro.params, ro.lo, ro.hi, ro.normalize,
-                    [&](int a) { return normal_slot<T>(ro.seed, gid, pstep, a); });
+                    [&](int a) { return normal_slot<T>(ro.seed, gid, pstep, a); }, ro.shape);
     if (active) {
       const PolicyStage<T>& ps = policy_stage<T>(s);
       for (int j = tl.lane; j < kObsDim3d; j += LANES) ro.obs[(size_t)e * kObsDim3d + j] = ps.obs[j];

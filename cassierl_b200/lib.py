@@ -18,6 +18,7 @@ MODE3D_TORQUE, MODE3D_PD = 0, 1
 AUTO_RESET_3D, TERMINAL_OBS_3D = 1, 8
 OBS_DIM_3D = 45
 POLICY_PARAMS_3D = 2868
+POLICY_MAX_LAYERS_3D, POLICY_MAX_WIDTH_3D = 4, 256
 F32, F64 = 32, 64
 
 # every symbol include/cassie2d.h declares
@@ -37,7 +38,8 @@ BATCH3D_SYMBOLS = ["Cassie3dGetLastError", "Cassie3dBatchCreate", "Cassie3dBatch
                    "Cassie3dBatchSetState", "Cassie3dBatchGetState", "Cassie3dBatchGetWarmStart", "Cassie3dBatchSetWarmStart",
                    "Cassie3dBatchStep", "Cassie3dBatchStepHost", "Cassie3dBatchGetStats", "Cassie3dBatchGetResets",
                    "Cassie3dBatchSetPdGains", "Cassie3dBatchEnvStep", "Cassie3dBatchEnvStepHost", "Cassie3dBatchEnvReset",
-                   "Cassie3dBatchObserve", "Cassie3dBatchGetEpisodeLengths", "Cassie3dBatchRollout", "Cassie3dBatchActionBox",
+                   "Cassie3dBatchObserve", "Cassie3dBatchGetEpisodeLengths", "Cassie3dBatchRollout", "Cassie3dBatchRolloutMlp",
+                   "Cassie3dBatchActionBox",
                    "Cassie3dBatchDiscountedReturns", "Cassie3dBatchBaselineMoments", "Cassie3dBatchAdvantages"]
 
 _lib = None
@@ -131,6 +133,8 @@ def load():
     L.Cassie3dBatchObserve.argtypes = [vp, vp, vp]
     L.Cassie3dBatchGetEpisodeLengths.argtypes = [vp, vp, vp]
     L.Cassie3dBatchRollout.argtypes = [vp, ci, vp, ci, ci, ci, ci, ci, ct.c_ulonglong, ct.c_uint, vp, vp, vp, vp, vp, vp]
+    L.Cassie3dBatchRolloutMlp.argtypes = [vp, ci, ci, i32p, vp, ci, ci, ci, ci, ci, ct.c_ulonglong, ct.c_uint, vp, vp, vp, vp,
+                                          vp, vp]
     L.Cassie3dBatchActionBox.argtypes = [vp, ci, ct.POINTER(cd), ct.POINTER(cd)]
     L.Cassie3dBatchDiscountedReturns.argtypes = [vp, vp, vp, vp, cd, ci, vp, vp]
     L.Cassie3dBatchBaselineMoments.argtypes = [vp, vp, vp, vp, vp, ci, vp, vp, vp]

@@ -1,8 +1,8 @@
 """Rollout collection for the reference's TRPO launcher (rllab/envs/trpo_cassie.py:13-55), batched:
 GaussianMLPPolicy(hidden_sizes=(32, 32)) + normalize(Cassie2dEnv) + rollout(max_path_length), fused in
 one CUDA kernel per T policy steps (csrc/rollout_kernels.cuh); RolloutCollector3d does the same on the 3-D stand env
-(csrc/tree_rollout.cuh, one launch pass per policy step).  Paths come back in rllab's dict layout
-(SURVEY App. E): observations[T,odim], actions[T,adim] (raw policy outputs), rewards[T],
+(csrc/tree_rollout.cuh, one launch pass per policy step) for any hidden_sizes of 1 to 4 layers up to 256 wide.
+Paths come back in rllab's dict layout (SURVEY App. E): observations[T,odim], actions[T,adim] (raw policy outputs), rewards[T],
 agent_infos{mean, log_std}, env_infos{}.  The TRPO update itself is rllab's and out of scope.
 """
 import math
@@ -13,34 +13,44 @@ import torch
 from . import lib as _lib
 from .envs import ACTION_DIM, MODE_BY_NAME, OBS_DIM, Cassie2dBatch, _stream_ptr
 
-HIDDEN = 32
+DEFAULT_HIDDEN_SIZES = (32, 32)   # trpo_cassie.py:21
 
 
-def n_params(obs_dim, act_dim):
-    return obs_dim * HIDDEN + HIDDEN + HIDDEN * HIDDEN + HIDDEN + HIDDEN * act_dim + act_dim + act_dim
+def n_params(obs_dim, act_dim, hidden_sizes=DEFAULT_HIDDEN_SIZES):
+    """length of GaussianMLPPolicy.flat: (in + 1) out per dense layer, plus log_std"""
+    n, fi = 0, obs_dim
+    for fo in tuple(hidden_sizes) + (act_dim,):
+        n += fi * fo + fo
+        fi = fo
+    return n + act_dim
 
 
 class GaussianMLPPolicy:
     """Parameter container with rllab's conventions: Lasagne DenseLayer weights W[in, out] (y = x W + b),
-    Glorot-uniform W, zero b, tanh hidden layers, linear mean head, state-independent log_std initialised
-    to log(init_std) (trpo_cassie.py:21-27: hidden_sizes=(32, 32), init_std=2.0).  `flat` is the vector
-    rllab's get_param_values() returns: W1 b1 W2 b2 W3 b3 log_std."""
+    Glorot-uniform W, zero b, tanh hidden layers of `hidden_sizes` units, linear mean head, state-independent log_std
+    initialised to log(init_std) (trpo_cassie.py:21-27: hidden_sizes=(32, 32), init_std=2.0; vpg_cassie.py uses
+    (128, 128)).  `flat` is the vector rllab's get_param_values() returns: W1 b1 W2 b2 ... W(L+1) b(L+1) log_std.
+    The planar collector takes (32, 32) only; RolloutCollector3d takes 1 to 4 hidden layers of 1 to 256 units."""
 
-    def __init__(self, obs_dim, act_dim, init_std=2.0, seed=1, device="cuda", dtype=torch.float32):
+    def __init__(self, obs_dim, act_dim, init_std=2.0, seed=1, device="cuda", dtype=torch.float32, *,
+                 hidden_sizes=DEFAULT_HIDDEN_SIZES):
+        self.hidden_sizes = tuple(int(h) for h in hidden_sizes)
         g = torch.Generator().manual_seed(seed)
+        widths = (obs_dim,) + self.hidden_sizes + (act_dim,)
         parts = []
-        for fi, fo in ((obs_dim, HIDDEN), (HIDDEN, HIDDEN), (HIDDEN, act_dim)):
+        for fi, fo in zip(widths[:-1], widths[1:]):
             lim = math.sqrt(6.0 / (fi + fo))
             parts += [(torch.rand(fi, fo, generator=g, dtype=torch.float64) * 2 - 1) * lim, torch.zeros(fo, dtype=torch.float64)]
         parts.append(torch.full((act_dim,), math.log(init_std), dtype=torch.float64))
         self.obs_dim, self.act_dim = obs_dim, act_dim
         self.flat = torch.cat([p.reshape(-1) for p in parts]).to(dtype=dtype, device=device).contiguous()
-        assert self.flat.numel() == n_params(obs_dim, act_dim)
+        assert self.flat.numel() == n_params(obs_dim, act_dim, self.hidden_sizes)
 
     def unpack(self, flat=None):
+        """[W1, b1, ..., W(L+1), b(L+1), log_std], views of `flat`"""
         f = self.flat if flat is None else flat
-        o, a, h = self.obs_dim, self.act_dim, HIDDEN
-        sizes = [(o, h), (h,), (h, h), (h,), (h, a), (a,), (a,)]
+        widths = (self.obs_dim,) + self.hidden_sizes + (self.act_dim,)
+        sizes = [s for fi, fo in zip(widths[:-1], widths[1:]) for s in ((fi, fo), (fo,))] + [(self.act_dim,)]
         out, k = [], 0
         for s in sizes:
             n = int(np.prod(s)); out.append(f[k:k + n].reshape(s)); k += n
@@ -48,14 +58,15 @@ class GaussianMLPPolicy:
 
     def mean(self, obs):
         """plain PyTorch reference of the kernel's forward pass (used by the tests)"""
-        W1, b1, W2, b2, W3, b3, _ = self.unpack()
-        h = torch.tanh(obs @ W1 + b1)
-        h = torch.tanh(h @ W2 + b2)
-        return h @ W3 + b3
+        p = self.unpack()
+        h = obs
+        for i in range(0, len(p) - 3, 2):
+            h = torch.tanh(h @ p[i] + p[i + 1])
+        return h @ p[-3] + p[-2]
 
     @property
     def log_std(self):
-        return self.unpack()[6]
+        return self.unpack()[-1]
 
 
 class _PathSampler:
@@ -186,8 +197,9 @@ class RolloutCollector(_PathSampler):
 
 
 class RolloutCollector3d(_PathSampler):
-    """The planar collector's interface on the 3-D stand env (include/cassie3d.h, Cassie3dBatchRollout):
-    GaussianMLPPolicy(45, 10) + normalize(Cassie3dBatchEnv) + rollout(max_path_length).  `collect(policy, T)` enqueues
+    """The planar collector's interface on the 3-D stand env (include/cassie3d.h, Cassie3dBatchRolloutMlp):
+    GaussianMLPPolicy(45, 10, hidden_sizes=...) + normalize(Cassie3dBatchEnv) + rollout(max_path_length), the policy
+    taking 1 to 4 hidden layers of 1 to 256 units.  `collect(policy, T)` enqueues
     one launch pass per policy step (the policy forward, the noise and the action map are fused into the env step) and
     returns the same dict as RolloutCollector.collect; dones are path codes: 1 terminated (fell or diverged), 2 cut at
     max_path_length.  Episodes continue across collect() calls."""
@@ -228,10 +240,11 @@ class RolloutCollector3d(_PathSampler):
         with torch.cuda.device(b.device):
             # where each env's current path stands: the in-path index of this batch's first samples (baseline features)
             self._check(b.L.Cassie3dBatchGetEpisodeLengths(b.h, self._path_start.data_ptr(), _stream_ptr()), "GetEpisodeLengths")
-            self._check(b.L.Cassie3dBatchRollout(
-                b.h, self.mode, p.data_ptr(), p.numel(), int(T), self.n_substeps, self.max_path_length, int(self.normalize),
-                self.seed, self.env0, self.obs.data_ptr(), self.act.data_ptr(), self.mean.data_ptr(), self.rew.data_ptr(),
-                self.done.data_ptr(), _stream_ptr()), "Rollout")
+            hs = policy.hidden_sizes
+            self._check(b.L.Cassie3dBatchRolloutMlp(
+                b.h, self.mode, len(hs), (_lib.ct.c_int32 * len(hs))(*hs), p.data_ptr(), p.numel(), int(T), self.n_substeps,
+                self.max_path_length, int(self.normalize), self.seed, self.env0, self.obs.data_ptr(), self.act.data_ptr(),
+                self.mean.data_ptr(), self.rew.data_ptr(), self.done.data_ptr(), _stream_ptr()), "Rollout")
         return dict(observations=self.obs, actions=self.act, means=self.mean, rewards=self.rew, dones=self.done)
 
     def discounted_returns(self, gamma=0.99, tail=None):

@@ -96,17 +96,18 @@ int Cassie3dBatchObserve(Cassie3dBatch* h, void* obs, void* stream);
 int Cassie3dBatchGetEpisodeLengths(Cassie3dBatch* h, int32_t* ep_len, void* stream);
 
 /* ---- rollout collection on the stand-task env (the planar Cassie2dBatchRollout's counterpart): rllab's BatchSampler
- * with GaussianMLPPolicy(hidden_sizes=(32, 32)) and normalize(env), n_policy_steps policy steps of every env, enqueued
- * on `stream` without a host synchronisation (one or two launches per policy step).
+ * with GaussianMLPPolicy(hidden_sizes) and normalize(env), n_policy_steps policy steps of every env, enqueued on
+ * `stream` without a host synchronisation (one or two launches per policy step).
  *
- * Per env and policy step k: obs[k] = the observation of the current state; mean[k] = tanh MLP 45 -> 32 -> 32 -> 10 with
- * a linear head, params_dev = rllab's flat vector W1 b1 W2 b2 W3 b3 log_std (real, W stored [in][out],
- * CASSIE3D_POLICY_PARAMS entries); action[k] = mean + exp(log_std) * eps, the raw policy output rllab stores; the env
- * action = lb + (action + 1) / 2 (ub - lb) clipped to [lb, ub] with normalize != 0, else action clipped; then
- * n_substeps >= 1 simulator steps and the EnvStep epilogue with auto-reset: reward[k] (its action term on the env
- * action), done[k] in path codes 1 = terminated (fell or diverged; a diverged env's reward is 0), 2 = cut because the
- * episode length reached max_path_length > 0, else 0.  Episodes continue across calls; the episode lengths are
- * EnvStep's (GetEpisodeLengths).
+ * Per env and policy step k: obs[k] = the observation of the current state; mean[k] = tanh MLP 45 -> h1 -> ... -> hL ->
+ * 10 with a linear head, hidden_sizes = (h1, ..., hL) (host int32 [n_hidden]), 1 <= L <= CASSIE3D_POLICY_MAX_LAYERS,
+ * 1 <= h <= CASSIE3D_POLICY_MAX_WIDTH; params_dev = rllab's flat vector W1 b1 W2 b2 ... W(L+1) b(L+1) log_std (real,
+ * W stored [in][out]), n_params = its length, sum over layers of (in + 1) out, plus 10; action[k] = mean + exp(log_std)
+ * * eps, the raw policy output rllab stores; the env action = lb + (action + 1) / 2 (ub - lb) clipped to [lb, ub] with
+ * normalize != 0, else action clipped; then n_substeps >= 1 simulator steps and the EnvStep epilogue with auto-reset:
+ * reward[k] (its action term on the env action), done[k] in path codes 1 = terminated (fell or diverged; a diverged env's
+ * reward is 0), 2 = cut because the episode length reached max_path_length > 0, else 0.  Episodes continue across calls;
+ * the episode lengths are EnvStep's (GetEpisodeLengths).
  *
  * Buffers (device): obs real [T][n][CASSIE3D_OBS_DIM], action / mean real [T][n][nu], reward real [T][n], done uint8
  * [T][n], T = n_policy_steps.
@@ -115,7 +116,16 @@ int Cassie3dBatchGetEpisodeLengths(Cassie3dBatch* h, int32_t* ep_len, void* stre
  * Noise: eps of action a = Box-Muller on Philox4x32-10 with key = seed (low word first) and counter {first_global_env +
  * e, step, a / 4, 0}, step = the env's rollout policy-step counter (0 at Create, advanced by Rollout only, never reset):
  * actions 0..7 are the two pairs of blocks 0 and 1 as in the planar rollout, actions 8 and 9 the first pair of block 2.
- * A batch holding global envs [first_global_env, first_global_env + n) therefore draws what one large batch would. */
+ * A batch holding global envs [first_global_env, first_global_env + n) therefore draws what one large batch would, and
+ * the noise does not depend on hidden_sizes.
+ * Returns -1 (Cassie3dGetLastError) for a null pointer, an unknown mode, n_substeps < 1, max_path_length <= 0, a shape
+ * outside the limits or an n_params that is not the shape's. */
+enum { CASSIE3D_POLICY_MAX_LAYERS = 4, CASSIE3D_POLICY_MAX_WIDTH = 256 };
+int Cassie3dBatchRolloutMlp(Cassie3dBatch* h, int mode, int n_hidden, const int32_t* hidden_sizes, const void* params_dev,
+                            int n_params, int n_policy_steps, int n_substeps, int max_path_length, int normalize,
+                            unsigned long long seed, unsigned int first_global_env, void* obs_dev, void* action_dev,
+                            void* mean_dev, void* reward_dev, uint8_t* done_dev, void* stream);
+/* RolloutMlp with hidden_sizes = (32, 32), the reference's TRPO launcher's: CASSIE3D_POLICY_PARAMS entries */
 enum { CASSIE3D_POLICY_PARAMS = 2868 };
 int Cassie3dBatchRollout(Cassie3dBatch* h, int mode, const void* params_dev, int n_params, int n_policy_steps,
                          int n_substeps, int max_path_length, int normalize, unsigned long long seed,

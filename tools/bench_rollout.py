@@ -3,13 +3,16 @@ sampler-side pre-processing (returns, LinearFeatureBaseline fit, GAE advantages)
 bench (bench.py); prints one JSON line for profiles/.
 
   python tools/bench_rollout.py [--envs N] [--T T] [--mode PD|OSC|TORQUE]
-  python tools/bench_rollout.py --model 3d [--envs N] [--T T] [--mode PD|TORQUE]      # the 3-D stand env
+  python tools/bench_rollout.py --model 3d [--envs N] [--T T] [--mode PD|TORQUE] [--hidden 128,128]   # the 3-D stand env
   python -m torch.distributed.run --nproc-per-node G ... tools/bench_rollout.py     # N envs PER GPU, one rank per GPU
 
---model 3d (RolloutCollector3d, default 8192 envs per GPU, T = 20, PD) also times, in the same process and alternated
-twice, the loop a user would otherwise write on Cassie3dBatchEnv (PyTorch policy forward, randn, affine map, clamp,
-EnvStep) and EnvStep alone on pre-generated actions (an upper bound for the fused collect), and reports the rollout and
-env kernels' launch resources read from a torch.profiler trace, with the card's name and power limit.
+--model 3d (RolloutCollector3d, default 8192 envs per GPU, T = 20, PD; --hidden the policy's hidden_sizes, default
+32,32) also sweeps hidden_sizes (32, 32) (64, 64) (128, 128) (256, 256): at each shape it times, in the same process and
+alternated twice, the fused collect, the loop a user would otherwise write on Cassie3dBatchEnv (PyTorch policy forward,
+randn, affine map, clamp, EnvStep) and EnvStep alone on pre-generated actions (an upper bound for the fused collect).  It
+reports the rollout and env kernels' launch resources read from a torch.profiler trace, with the card's name and power
+limit.  The sweep spans the reference launchers' (32, 32) and (128, 128) up to the widest shape the kernel takes, whose
+fp32 weights (318 KB) no longer fit in L1.
 
 Multi-GPU (SURVEY 8e): envs are sharded by global env id (Philox streams and phases do not depend on G), there is no
 collective inside a rollout; after it, NCCL all-reduces the rollout statistics (cassierl_b200.parallel.RolloutStats) and
@@ -38,7 +41,11 @@ p.add_argument("--T", type=int, default=20, help="policy steps per collect() (10
 p.add_argument("--reps", type=int, default=5)
 p.add_argument("--mode", default="PD", choices=["PD", "OSC", "TORQUE"])
 p.add_argument("--task", default="stand", choices=["stand", "imitate"])
+p.add_argument("--hidden", default="32,32", help="the policy's hidden_sizes, comma-separated (the planar rollout: 32,32)")
 a = p.parse_args()
+hidden = tuple(int(h) for h in a.hidden.split(","))
+if a.model == "2d" and hidden != (32, 32):
+    p.error("the planar rollout takes hidden_sizes (32, 32) only")
 if a.envs is None:
     a.envs = 8192 if a.model == "3d" else 16384
 if a.model == "3d" and a.mode == "OSC":
@@ -56,7 +63,7 @@ if a.model == "3d":
                              first_global_env=rank * a.envs)
 else:
     col = RolloutCollector(a.envs, device=local, task=a.task, control_mode=a.mode, max_path_length=1000, first_global_env=rank * a.envs)
-pol = GaussianMLPPolicy(col.obs_dim, col.act_dim, device=dev)
+pol = GaussianMLPPolicy(col.obs_dim, col.act_dim, device=dev, hidden_sizes=hidden)
 if world > 1:
     dist.broadcast(pol.flat, src=0)            # the learner's parameters (8.5 kB), once per iteration
 col.collect(pol, a.T)                      # warm-up (also sizes the buffers)
@@ -120,53 +127,61 @@ def kernel_resources(fns, names):
     return out
 
 
+SWEEP_3D = ((32, 32), (64, 64), (128, 128), (256, 256))
+
+
 def compare_3d():
-    """(a) the fused collect, (b) the unfused loop on Cassie3dBatchEnv, (c) EnvStep alone on pre-generated actions;
-    same envs, policy and T, alternated twice, CUDA-event times (median of --reps each)"""
+    """at each shape of SWEEP_3D: (a) the fused collect, (b) the unfused loop on Cassie3dBatchEnv, (c) EnvStep alone on
+    pre-generated actions; same envs and T, alternated twice, CUDA-event times (median of --reps each)"""
     from cassierl_b200.envs3d import Cassie3dBatchEnv
     env = Cassie3dBatchEnv(a.envs, device=local, control_mode=col.control_mode, auto_reset=True, max_path_length=1000)
     env.reset()
     n, T = a.envs, a.T
     lo, hi = (torch.tensor(x, dtype=env.batch.dtype, device=dev) for x in col.action_space)
-    W1, b1, W2, b2, W3, b3, log_std = pol.unpack()
-    std = log_std.exp()
     mk = lambda *sh, dt=env.batch.dtype: torch.empty(sh, dtype=dt, device=dev)
     bo, ba, bm, br, bd = mk(T, n, 45), mk(T, n, 10), mk(T, n, 10), mk(T, n), mk(T, n, dt=torch.uint8)
     state = {"obs": env.observe().clone()}
-
-    def unfused():
-        o = state["obs"]
-        for k in range(T):
-            h = torch.tanh(o @ W1 + b1)
-            h = torch.tanh(h @ W2 + b2)
-            mean = h @ W3 + b3
-            act = mean + std * torch.randn_like(mean)
-            x = (lo + (act + 1.0) * 0.5 * (hi - lo)).clamp(lo, hi)
-            bo[k].copy_(o); ba[k].copy_(act); bm[k].copy_(mean)
-            o, r, d = env.step(x)
-            br[k].copy_(r); bd[k].copy_(d)
-        state["obs"] = o
-
     pre = (lo + (torch.rand(T, n, 10, device=dev, dtype=env.batch.dtype)) * (hi - lo)).contiguous()
 
     def env_only():
         for k in range(T):
             env.step(pre[k])
 
-    unfused(); env_only(); torch.cuda.synchronize()                      # warm-up of every shape
-    runs = {"fused_collect": [], "unfused_loop": [], "env_step_only": []}
-    for _ in range(2):
-        runs["fused_collect"].append(timed(lambda: col.collect(pol, T), a.reps))
-        runs["unfused_loop"].append(timed(unfused, a.reps))
-        runs["env_step_only"].append(timed(env_only, a.reps))
-    res = kernel_resources([lambda: col.collect(pol, 2), lambda: env.step(pre[0])], ["k_tree_rollout_step", "k_tree_env_step"])
-    best = {k: min(v) for k, v in runs.items()}
-    env.terminate()
-    return {"ms_per_collect": runs,
-            "env_steps_per_s": {k: [n * T * 10 / (x * 1e-3) for x in v] for k, v in runs.items()},
+    sweep, res = {}, None
+    for shape in SWEEP_3D:
+        sp = GaussianMLPPolicy(col.obs_dim, col.act_dim, device=dev, hidden_sizes=shape)
+        layers = sp.unpack()
+        std = layers[-1].exp()
+
+        def unfused():
+            o = state["obs"]
+            for k in range(T):
+                h = o
+                for i in range(0, len(layers) - 3, 2):
+                    h = torch.tanh(h @ layers[i] + layers[i + 1])
+                mean = h @ layers[-3] + layers[-2]
+                act = mean + std * torch.randn_like(mean)
+                x = (lo + (act + 1.0) * 0.5 * (hi - lo)).clamp(lo, hi)
+                bo[k].copy_(o); ba[k].copy_(act); bm[k].copy_(mean)
+                o, r, d = env.step(x)
+                br[k].copy_(r); bd[k].copy_(d)
+            state["obs"] = o
+
+        col.collect(sp, T); unfused(); env_only(); torch.cuda.synchronize()      # warm-up of every shape
+        runs = {"fused_collect": [], "unfused_loop": [], "env_step_only": []}
+        for _ in range(2):
+            runs["fused_collect"].append(timed(lambda: col.collect(sp, T), a.reps))
+            runs["unfused_loop"].append(timed(unfused, a.reps))
+            runs["env_step_only"].append(timed(env_only, a.reps))
+        if res is None:
+            res = kernel_resources([lambda: col.collect(sp, 2), lambda: env.step(pre[0])], ["k_tree_rollout_step", "k_tree_env_step"])
+        best = {k: min(v) for k, v in runs.items()}
+        sweep["x".join(map(str, shape))] = {
+            "ms_per_collect": runs, "env_steps_per_s": {k: [n * T * 10 / (x * 1e-3) for x in v] for k, v in runs.items()},
             "fused_vs_env_step_only": best["fused_collect"] / best["env_step_only"] - 1.0,
-            "fused_vs_unfused": best["fused_collect"] / best["unfused_loop"] - 1.0,
-            "kernels": res, "card": card()}
+            "fused_vs_unfused": best["fused_collect"] / best["unfused_loop"] - 1.0}
+    env.terminate()
+    return {"hidden_sizes_sweep": sweep, "kernels": res, "card": card()}
 
 
 ms_collect = timed(lambda: col.collect(pol, a.T), a.reps)
@@ -219,8 +234,8 @@ if a.model == "3d":
     st = col.batch.stats().double()   # [n, 4]: constraint rows, contacts, PGS sweeps, contacts dropped
     if rank == 0:
         print(json.dumps({
-            "workload": "rollout: GaussianMLPPolicy(45->32->32->10) + %s action space + cassie3d stand env, %d envs per GPU x %d GPUs x %d policy steps x 10 sim steps"
-                        % (col.control_mode, a.envs, world, a.T),
+            "workload": "rollout: GaussianMLPPolicy(45->%s->10) + %s action space + cassie3d stand env, %d envs per GPU x %d GPUs x %d policy steps x 10 sim steps"
+                        % ("->".join(map(str, hidden)), col.control_mode, a.envs, world, a.T),
             "n_gpus": world, "collect_ms": ms_collect, "env_steps_per_s": n_total * a.T * 10 / (ms_collect * 1e-3),
             "policy_steps_per_s": n_total * a.T / (ms_collect * 1e-3),
             "env_steps_per_s_with_overlapped_gather": (n_total * a.T * 10 / (gather["collect_with_overlapped_gather_ms"] * 1e-3)) if world > 1 else None,
