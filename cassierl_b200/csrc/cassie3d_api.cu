@@ -1,4 +1,5 @@
 // C-ABI of the batched 3-D step path (include/cassie3d.h).  Host glue only: the arithmetic is tree_engine.cuh.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -58,6 +59,7 @@ struct Cassie3dBatch {
   int32_t* ep_len = nullptr;  // [n] policy steps since the env's last reset (EnvStep)
   int32_t* policy_step = nullptr;   // [n] Philox step counter of Rollout: zero at Create, advanced by Rollout only
   void* d_act_env = nullptr;  // [n][nu] the mapped, clipped action of Rollout's current policy step
+  void* d_ou = nullptr;       // [n][nu] OU state of RolloutOU: zero at Create, reset to mu at every path start
   std::vector<double> kp, kd; // PD gains of the env's kActPd action space, per motor
   cudaStream_t own_stream = nullptr;
   size_t rs() const { return precision == 64 ? 8 : 4; }
@@ -92,7 +94,8 @@ int setup(Cassie3dBatch* h, TreeBatchView<T>& v) {
       dmalloc(h, &h->d_reset_qd, sizeof(T) * m.nv) || dmalloc(h, &h->d_action, sizeof(T) * n * m.nu) ||
       dmalloc(h, (void**)&h->d_done, n) || dmalloc(h, &h->d_obs, sizeof(T) * n * kObsDim3d) ||
       dmalloc(h, &h->d_reward, sizeof(T) * n) || dmalloc(h, (void**)&h->ep_len, sizeof(int32_t) * n) ||
-      dmalloc(h, (void**)&h->policy_step, sizeof(int32_t) * n) || dmalloc(h, &h->d_act_env, sizeof(T) * n * m.nu))
+      dmalloc(h, (void**)&h->policy_step, sizeof(int32_t) * n) || dmalloc(h, &h->d_act_env, sizeof(T) * n * m.nu) ||
+      dmalloc(h, &h->d_ou, sizeof(T) * n * m.nu))
     return -1;
   return 0;
 }
@@ -138,10 +141,15 @@ int env_step(Cassie3dBatch* h, int mode, const void* action, int n_sub, int max_
   return 0;
 }
 
+// the OUStrategy of RolloutOU (kPolicyOu3d); unused by the Gaussian kind
+struct OuArgs {
+  double mu, theta, sigma;
+};
+
 template <typename T>
-int rollout(Cassie3dBatch* h, int mode, const PolicyShape3d& shape, const void* params, int T_steps, int n_sub,
-            int max_path_length, int normalize, unsigned long long seed, unsigned int env0, void* obs, void* act, void* mean,
-            void* reward, uint8_t* done, cudaStream_t s) {
+int rollout(Cassie3dBatch* h, int mode, const PolicyShape3d& shape, int kind, const OuArgs& ou, const void* params, int T_steps,
+            int n_sub, int max_path_length, int normalize, unsigned long long seed, unsigned int env0, void* obs, void* act,
+            void* mean, void* reward, uint8_t* done, cudaStream_t s) {
   const size_t n = (size_t)h->n, nu = (size_t)h->model.nu;
   TreeStepArgs a;
   a.action = nullptr; a.n_sub = n_sub; a.z_done = 0; a.auto_reset = 1; a.done = nullptr;
@@ -158,6 +166,7 @@ int rollout(Cassie3dBatch* h, int mode, const PolicyShape3d& shape, const void* 
   action_box(h->model, mode, lo, hi);
   for (int i = 0; i < kMaxAct; i++) { ro.lo[i] = (T)lo[i]; ro.hi[i] = (T)hi[i]; }
   ro.params = (const T*)params; ro.shape = shape; ro.normalize = normalize; ro.seed = seed; ro.env0 = env0;
+  ro.kind = kind; ro.ou_mu = (T)ou.mu; ro.ou_theta = (T)ou.theta; ro.ou_sigma = (T)ou.sigma; ro.ou = (T*)h->d_ou;
   ro.policy_step = h->policy_step; ro.act_env = (T*)h->d_act_env;
   for (int k = 0; k < T_steps; k++) {   // one launch pass per policy step, no host synchronisation in between
     ro.obs = (T*)obs + (size_t)k * n * kObsDim3d;
@@ -182,6 +191,33 @@ int check_env_step(Cassie3dBatch* h, int mode, const void* action, int n_substep
   if (!action) return fail3("EnvStep needs an action");
   if (n_substeps < 1) return fail3("n_substeps must be at least 1");
   if (flags & ~(CASSIE3D_AUTO_RESET | CASSIE3D_TERMINAL_OBS)) return fail3("unknown flag bits");
+  return 0;
+}
+
+// the checks RolloutMlp and RolloutOU share; fills `shape`
+int check_rollout(Cassie3dBatch* h, int mode, int n_hidden, const int32_t* hidden_sizes, int kind, const void* params_dev,
+                  int n_params, int n_policy_steps, int n_substeps, int max_path_length, void* obs_dev, void* action_dev,
+                  void* mean_dev, void* reward_dev, uint8_t* done_dev, PolicyShape3d* shape) {
+  if (!h || !hidden_sizes || !params_dev || !obs_dev || !action_dev || !mean_dev || !reward_dev || !done_dev)
+    return fail3("null argument");
+  if (mode != CASSIE3D_MODE_TORQUE && mode != CASSIE3D_MODE_PD) return fail3("mode must be CASSIE3D_MODE_TORQUE or CASSIE3D_MODE_PD");
+  if (n_policy_steps < 0) return fail3("n_policy_steps must not be negative");
+  if (n_substeps < 1) return fail3("n_substeps must be at least 1");
+  if (max_path_length <= 0) return fail3("max_path_length must be positive");
+  if (n_hidden < 1 || n_hidden > kPolicyMaxLayers3d)
+    return fail3("n_hidden is " + std::to_string(n_hidden) + ", the policy takes 1 to " + std::to_string(kPolicyMaxLayers3d) + " hidden layers");
+  *shape = PolicyShape3d{n_hidden, {0, 0, 0, 0}};
+  for (int l = 0; l < n_hidden; l++) {
+    if (hidden_sizes[l] < 1 || hidden_sizes[l] > kPolicyMaxWidth3d)
+      return fail3("hidden_sizes[" + std::to_string(l) + "] is " + std::to_string(hidden_sizes[l]) + ", a hidden layer has 1 to " +
+                   std::to_string(kPolicyMaxWidth3d) + " units");
+    shape->width[l] = hidden_sizes[l];
+  }
+  const int want = policy_params3d(*shape, kind);
+  if (n_params != want)
+    return fail3("policy parameter vector has " + std::to_string(n_params) + " entries, expected " + std::to_string(want) +
+                 (kind == kPolicyOu3d ? " (DeterministicMLPPolicy: no log_std)" : ""));
+  if (h->model.nu != kPolicyAct3d) return fail3("the policy has " + std::to_string(kPolicyAct3d) + " actions, the model " + std::to_string(h->model.nu) + " motors");
   return 0;
 }
 }  // namespace
@@ -428,31 +464,39 @@ int Cassie3dBatchRolloutMlp(Cassie3dBatch* h, int mode, int n_hidden, const int3
                             int n_params, int n_policy_steps, int n_substeps, int max_path_length, int normalize,
                             unsigned long long seed, unsigned int first_global_env, void* obs_dev, void* action_dev,
                             void* mean_dev, void* reward_dev, uint8_t* done_dev, void* stream) {
-  if (!h || !hidden_sizes || !params_dev || !obs_dev || !action_dev || !mean_dev || !reward_dev || !done_dev)
-    return fail3("null argument");
-  if (mode != CASSIE3D_MODE_TORQUE && mode != CASSIE3D_MODE_PD) return fail3("mode must be CASSIE3D_MODE_TORQUE or CASSIE3D_MODE_PD");
-  if (n_policy_steps < 0) return fail3("n_policy_steps must not be negative");
-  if (n_substeps < 1) return fail3("n_substeps must be at least 1");
-  if (max_path_length <= 0) return fail3("max_path_length must be positive");
-  if (n_hidden < 1 || n_hidden > kPolicyMaxLayers3d)
-    return fail3("n_hidden is " + std::to_string(n_hidden) + ", the policy takes 1 to " + std::to_string(kPolicyMaxLayers3d) + " hidden layers");
-  PolicyShape3d shape = {n_hidden, {0, 0, 0, 0}};
-  for (int l = 0; l < n_hidden; l++) {
-    if (hidden_sizes[l] < 1 || hidden_sizes[l] > kPolicyMaxWidth3d)
-      return fail3("hidden_sizes[" + std::to_string(l) + "] is " + std::to_string(hidden_sizes[l]) + ", a hidden layer has 1 to " +
-                   std::to_string(kPolicyMaxWidth3d) + " units");
-    shape.width[l] = hidden_sizes[l];
-  }
-  const int want = policy_params3d(shape);
-  if (n_params != want)
-    return fail3("policy parameter vector has " + std::to_string(n_params) + " entries, expected " + std::to_string(want));
-  if (h->model.nu != kPolicyAct3d) return fail3("the policy has " + std::to_string(kPolicyAct3d) + " actions, the model " + std::to_string(h->model.nu) + " motors");
+  PolicyShape3d shape;
+  if (check_rollout(h, mode, n_hidden, hidden_sizes, kPolicyGaussian3d, params_dev, n_params, n_policy_steps, n_substeps,
+                    max_path_length, obs_dev, action_dev, mean_dev, reward_dev, done_dev, &shape))
+    return -1;
   DeviceGuard g(h->device);
   cudaStream_t s = (cudaStream_t)stream;
-  return DISPATCH3(h, rollout<float>(h, mode, shape, params_dev, n_policy_steps, n_substeps, max_path_length, normalize, seed,
-                                     first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s),
-                   rollout<double>(h, mode, shape, params_dev, n_policy_steps, n_substeps, max_path_length, normalize, seed,
-                                   first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s));
+  const OuArgs ou = {0, 0, 0};
+  return DISPATCH3(h, rollout<float>(h, mode, shape, kPolicyGaussian3d, ou, params_dev, n_policy_steps, n_substeps, max_path_length,
+                                     normalize, seed, first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s),
+                   rollout<double>(h, mode, shape, kPolicyGaussian3d, ou, params_dev, n_policy_steps, n_substeps, max_path_length,
+                                   normalize, seed, first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s));
+}
+
+int Cassie3dBatchRolloutOU(Cassie3dBatch* h, int mode, int n_hidden, const int32_t* hidden_sizes, const void* params_dev,
+                           int n_params, double ou_mu, double ou_theta, double ou_sigma, int n_policy_steps,
+                           int n_substeps, int max_path_length, int normalize, unsigned long long seed,
+                           unsigned int first_global_env, void* obs_dev, void* action_dev, void* mean_dev,
+                           void* reward_dev, uint8_t* done_dev, void* stream) {
+  PolicyShape3d shape;
+  if (check_rollout(h, mode, n_hidden, hidden_sizes, kPolicyOu3d, params_dev, n_params, n_policy_steps, n_substeps,
+                    max_path_length, obs_dev, action_dev, mean_dev, reward_dev, done_dev, &shape))
+    return -1;
+  if (!std::isfinite(ou_mu) || !std::isfinite(ou_theta) || !std::isfinite(ou_sigma))
+    return fail3("the OU parameters must be finite (mu " + std::to_string(ou_mu) + ", theta " + std::to_string(ou_theta) +
+                 ", sigma " + std::to_string(ou_sigma) + ")");
+  if (ou_sigma < 0) return fail3("ou_sigma is " + std::to_string(ou_sigma) + ", it must not be negative");
+  DeviceGuard g(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const OuArgs ou = {ou_mu, ou_theta, ou_sigma};
+  return DISPATCH3(h, rollout<float>(h, mode, shape, kPolicyOu3d, ou, params_dev, n_policy_steps, n_substeps, max_path_length,
+                                     normalize, seed, first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s),
+                   rollout<double>(h, mode, shape, kPolicyOu3d, ou, params_dev, n_policy_steps, n_substeps, max_path_length,
+                                   normalize, seed, first_global_env, obs_dev, action_dev, mean_dev, reward_dev, done_dev, s));
 }
 
 int Cassie3dBatchRollout(Cassie3dBatch* h, int mode, const void* params_dev, int n_params, int n_policy_steps,

@@ -210,15 +210,18 @@ k_tree_env_step(const __grid_constant__ TreeModel<T> m, const TreeBatchView<T> v
 template <typename T>
 struct TreeRolloutParams {
   T lo[kMaxAct], hi[kMaxAct];   // action box: ctrlrange (torque mode) or the motors' joint ranges (PD mode)
-  const T* params;              // [policy_params3d(shape)] GaussianMLPPolicy.flat
+  const T* params;              // [policy_params3d(shape, kind)] GaussianMLPPolicy.flat / DeterministicMLPPolicy.flat
   PolicyShape3d shape;          // hidden_sizes
+  int kind;                     // kPolicyGaussian3d, or kPolicyOu3d: DeterministicMLPPolicy + OUStrategy
+  T ou_mu, ou_theta, ou_sigma;  // OUStrategy (kPolicyOu3d)
+  T* ou;                        // [n][nu] OU state (kPolicyOu3d), advanced by the fast (or single) pass of active tiles
   int normalize;                // NormalizedEnv's affine map before the clip
   uint64_t seed;
   uint32_t env0;                // global id of this batch's env 0
   int32_t* policy_step;         // [n] Philox step counter, advanced by every finished policy step
   T* act_env;                   // [n][nu] the mapped, clipped action (the continuation pass reads it)
   T* obs;                       // [n][kObsDim3d] row k: the observation the policy saw
-  T* act;                       // [n][nu] raw policy output
+  T* act;                       // [n][nu] raw policy output (kPolicyOu3d: the clipped exploratory action)
   T* mean;                      // [n][nu]
   T* rew;                       // [n]
   uint8_t* done;                // [n] path codes: 1 terminated, 2 cut at max_path_length
@@ -227,7 +230,8 @@ struct TreeRolloutParams {
 // One policy step of Cassie3dBatchRollout: the passes of k_tree_env_step (same MODEs, physics and stand-task epilogue,
 // auto-reset always on), with the policy's prologue (tree_rollout.cuh) in MODE 0 / 1 instead of an action from the host.
 // The continuation pass re-reads the env action from ro.act_env.  The epilogue writes the path row: reward (its action
-// term on the env action), the done code in path codes, and advances policy_step.  A separate kernel, so that
+// term on the env action), the done code in path codes, and advances policy_step.  The policy kind (Gaussian, or
+// deterministic + OU for RolloutOU) is a kernel parameter like the widths.  A separate kernel, so that
 // k_tree_step and k_tree_env_step compile exactly as without it.
 template <typename T, int LANES, int ROWS, int CON, int MODE>
 __global__ void __launch_bounds__(kTreeMaxBlock)
@@ -260,8 +264,10 @@ k_tree_rollout_step(const __grid_constant__ TreeModel<T> m, const TreeBatchView<
   tl.sync();
   if (MODE != 2) {
     const uint32_t gid = ro.env0 + (uint32_t)e, pstep = (uint32_t)ro.policy_step[e];
+    // the OU state of env e: mirrored tiles (e_raw >= v.n) read it but must not advance it a second time
+    const OuStep3d<T> ou = {ro.ou_mu, ro.ou_theta, ro.ou_sigma, ro.ou + (size_t)e * nu, env.ep_len + e, active};
     policy_prologue(tl, m, s, ro.params, ro.lo, ro.hi, ro.normalize,
-                    [&](int a) { return normal_slot<T>(ro.seed, gid, pstep, a); }, ro.shape);
+                    [&](int a) { return normal_slot<T>(ro.seed, gid, pstep, a); }, ro.shape, ro.kind, ou);
     if (active) {
       const PolicyStage<T>& ps = policy_stage<T>(s);
       for (int j = tl.lane; j < kObsDim3d; j += LANES) ro.obs[(size_t)e * kObsDim3d + j] = ps.obs[j];

@@ -39,7 +39,7 @@ BATCH3D_SYMBOLS = ["Cassie3dGetLastError", "Cassie3dBatchCreate", "Cassie3dBatch
                    "Cassie3dBatchStep", "Cassie3dBatchStepHost", "Cassie3dBatchGetStats", "Cassie3dBatchGetResets",
                    "Cassie3dBatchSetPdGains", "Cassie3dBatchEnvStep", "Cassie3dBatchEnvStepHost", "Cassie3dBatchEnvReset",
                    "Cassie3dBatchObserve", "Cassie3dBatchGetEpisodeLengths", "Cassie3dBatchRollout", "Cassie3dBatchRolloutMlp",
-                   "Cassie3dBatchActionBox",
+                   "Cassie3dBatchRolloutOU", "Cassie3dBatchActionBox",
                    "Cassie3dBatchDiscountedReturns", "Cassie3dBatchBaselineMoments", "Cassie3dBatchAdvantages"]
 
 _lib = None
@@ -135,6 +135,8 @@ def load():
     L.Cassie3dBatchRollout.argtypes = [vp, ci, vp, ci, ci, ci, ci, ci, ct.c_ulonglong, ct.c_uint, vp, vp, vp, vp, vp, vp]
     L.Cassie3dBatchRolloutMlp.argtypes = [vp, ci, ci, i32p, vp, ci, ci, ci, ci, ci, ct.c_ulonglong, ct.c_uint, vp, vp, vp, vp,
                                           vp, vp]
+    L.Cassie3dBatchRolloutOU.argtypes = [vp, ci, ci, i32p, vp, ci, cd, cd, cd, ci, ci, ci, ci, ct.c_ulonglong, ct.c_uint, vp, vp,
+                                         vp, vp, vp, vp]
     L.Cassie3dBatchActionBox.argtypes = [vp, ci, ct.POINTER(cd), ct.POINTER(cd)]
     L.Cassie3dBatchDiscountedReturns.argtypes = [vp, vp, vp, vp, cd, ci, vp, vp]
     L.Cassie3dBatchBaselineMoments.argtypes = [vp, vp, vp, vp, vp, ci, vp, vp, vp]

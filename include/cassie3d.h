@@ -131,6 +131,25 @@ int Cassie3dBatchRollout(Cassie3dBatch* h, int mode, const void* params_dev, int
                          int n_substeps, int max_path_length, int normalize, unsigned long long seed,
                          unsigned int first_global_env, void* obs_dev, void* action_dev, void* mean_dev,
                          void* reward_dev, uint8_t* done_dev, void* stream);
+/* RolloutMlp with DDPG's sampler: rllab's DeterministicMLPPolicy(hidden_sizes) explored by OUStrategy(mu, theta, sigma).
+ *
+ * Per env and policy step k: mean[k] = tanh(b + x W) of a relu MLP 45 -> h1 -> ... -> hL -> 10 (same shape limits);
+ * params_dev = W1 b1 ... W(L+1) b(L+1) with NO log_std, n_params = the sum over layers of (in + 1) out.  OU state x
+ * (real [n][nu], kept in the handle across calls): at a path start (the env's episode length is 0: after Create,
+ * ResetAll, SetState, EnvReset or an auto-reset) x = ou_mu, as rllab's es.reset() after env.reset(); then
+ * x += ou_theta (ou_mu - x) + ou_sigma eps, eps the same standard normal of (seed, global env, step, action) RolloutMlp
+ * draws.  action[k] = clip(mean + x, -1, 1) with normalize != 0 (the box of normalize(env)), else clip(mean + x, lb, ub):
+ * the clipped exploratory action rllab's DDPG stores in its pool; the env action is mapped from it as in RolloutMlp.
+ * Every finished policy step advances x once.  The state is zero at Create and is not touched by the other calls, so a
+ * path already under way at the first RolloutOU call (e.g. run by RolloutMlp or EnvStep before) starts from x = 0, not
+ * mu.  Buffers, reward, done and the noise counter are RolloutMlp's.
+ * Returns -1 as RolloutMlp does, and for an n_params that is not the deterministic count (a Gaussian vector with its
+ * log_std included), a non-finite ou_mu, ou_theta or ou_sigma, or ou_sigma < 0. */
+int Cassie3dBatchRolloutOU(Cassie3dBatch* h, int mode, int n_hidden, const int32_t* hidden_sizes, const void* params_dev,
+                           int n_params, double ou_mu, double ou_theta, double ou_sigma, int n_policy_steps,
+                           int n_substeps, int max_path_length, int normalize, unsigned long long seed,
+                           unsigned int first_global_env, void* obs_dev, void* action_dev, void* mean_dev,
+                           void* reward_dev, uint8_t* done_dev, void* stream);
 /* host doubles [nu]: the action box Rollout maps into and clips to in `mode` */
 int Cassie3dBatchActionBox(Cassie3dBatch* h, int mode, double* lo, double* hi);
 /* sampler side of rllab's process_samples on Rollout's [T][n] buffers, as the planar calls of the same names:

@@ -4,6 +4,7 @@ bench (bench.py); prints one JSON line for profiles/.
 
   python tools/bench_rollout.py [--envs N] [--T T] [--mode PD|OSC|TORQUE]
   python tools/bench_rollout.py --model 3d [--envs N] [--T T] [--mode PD|TORQUE] [--hidden 128,128]   # the 3-D stand env
+  python tools/bench_rollout.py --model 3d --policy ou      # DDPG's sampler: DeterministicMLPPolicy + OUStrategy
   python -m torch.distributed.run --nproc-per-node G ... tools/bench_rollout.py     # N envs PER GPU, one rank per GPU
 
 --model 3d (RolloutCollector3d, default 8192 envs per GPU, T = 20, PD; --hidden the policy's hidden_sizes, default
@@ -13,6 +14,10 @@ randn, affine map, clamp, EnvStep) and EnvStep alone on pre-generated actions (a
 reports the rollout and env kernels' launch resources read from a torch.profiler trace, with the card's name and power
 limit.  The sweep spans the reference launchers' (32, 32) and (128, 128) up to the widest shape the kernel takes, whose
 fp32 weights (318 KB) no longer fit in L1.
+
+--policy ou (3-D only) adds DDPG's fused collect (DeterministicMLPPolicy + OUStrategy, Cassie3dBatchRolloutOU) to that
+alternation, at the reference launchers' (32, 32) and (128, 128) only, and times the sampler side of DDPG instead of
+returns + baseline + GAE: transitions() + ReplayPool.add + random_batch(256).
 
 Multi-GPU (SURVEY 8e): envs are sharded by global env id (Philox streams and phases do not depend on G), there is no
 collective inside a rollout; after it, NCCL all-reduces the rollout statistics (cassierl_b200.parallel.RolloutStats) and
@@ -32,7 +37,8 @@ import torch.distributed as dist
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from cassierl_b200 import parallel  # noqa: E402
-from cassierl_b200.rollout import GaussianMLPPolicy, RolloutCollector, RolloutCollector3d  # noqa: E402
+from cassierl_b200.rollout import (DeterministicMLPPolicy, GaussianMLPPolicy, OUStrategy, ReplayPool, RolloutCollector,  # noqa: E402
+                                   RolloutCollector3d)
 
 p = argparse.ArgumentParser()
 p.add_argument("--model", default="2d", choices=["2d", "3d"], help="planar (cassie2d) or 3-D (cassie3d stand env)")
@@ -42,6 +48,8 @@ p.add_argument("--reps", type=int, default=5)
 p.add_argument("--mode", default="PD", choices=["PD", "OSC", "TORQUE"])
 p.add_argument("--task", default="stand", choices=["stand", "imitate"])
 p.add_argument("--hidden", default="32,32", help="the policy's hidden_sizes, comma-separated (the planar rollout: 32,32)")
+p.add_argument("--policy", default="gaussian", choices=["gaussian", "ou"],
+               help="gaussian: GaussianMLPPolicy (TRPO / VPG); ou: DeterministicMLPPolicy + OUStrategy (DDPG), 3-D only")
 a = p.parse_args()
 hidden = tuple(int(h) for h in a.hidden.split(","))
 if a.model == "2d" and hidden != (32, 32):
@@ -50,6 +58,9 @@ if a.envs is None:
     a.envs = 8192 if a.model == "3d" else 16384
 if a.model == "3d" and a.mode == "OSC":
     p.error("the 3-D env offers PD and TORQUE")
+if a.model == "2d" and a.policy == "ou":
+    p.error("the planar rollout takes a GaussianMLPPolicy only")
+ou = a.policy == "ou"
 
 world = int(os.environ.get("WORLD_SIZE", "1")); rank = int(os.environ.get("RANK", "0")); local = int(os.environ.get("LOCAL_RANK", "0"))
 torch.cuda.set_device(local)
@@ -63,12 +74,25 @@ if a.model == "3d":
                              first_global_env=rank * a.envs)
 else:
     col = RolloutCollector(a.envs, device=local, task=a.task, control_mode=a.mode, max_path_length=1000, first_global_env=rank * a.envs)
-pol = GaussianMLPPolicy(col.obs_dim, col.act_dim, device=dev, hidden_sizes=hidden)
+pol = (DeterministicMLPPolicy if ou else GaussianMLPPolicy)(col.obs_dim, col.act_dim, device=dev, hidden_sizes=hidden)
+es = OUStrategy() if ou else None
 if world > 1:
     dist.broadcast(pol.flat, src=0)            # the learner's parameters (8.5 kB), once per iteration
-col.collect(pol, a.T)                      # warm-up (also sizes the buffers)
-ret = col.discounted_returns()
-col.fit_baseline(ret); col.advantages()
+pool = ReplayPool(1000000, col.obs_dim, col.act_dim, device=dev) if ou else None   # rllab DDPG's default pool size
+
+
+def sampler_side():
+    """what the sampler does with a collect: DDPG's pool rows, or TRPO's returns, baseline and advantages"""
+    if ou:
+        pool.add(col.transitions())
+        pool.random_batch(256)
+    else:
+        r = col.discounted_returns()
+        col.fit_baseline(r); col.advantages()
+
+
+col.collect(pol, a.T, es)                  # warm-up (also sizes the buffers)
+sampler_side()
 torch.cuda.synchronize()
 
 
@@ -127,12 +151,13 @@ def kernel_resources(fns, names):
     return out
 
 
-SWEEP_3D = ((32, 32), (64, 64), (128, 128), (256, 256))
+SWEEP_3D = ((32, 32), (128, 128)) if ou else ((32, 32), (64, 64), (128, 128), (256, 256))
 
 
 def compare_3d():
     """at each shape of SWEEP_3D: (a) the fused collect, (b) the unfused loop on Cassie3dBatchEnv, (c) EnvStep alone on
-    pre-generated actions; same envs and T, alternated twice, CUDA-event times (median of --reps each)"""
+    pre-generated actions, with --policy ou (d) the fused OU collect; same envs and T, alternated twice, CUDA-event times
+    (median of --reps each)"""
     from cassierl_b200.envs3d import Cassie3dBatchEnv
     env = Cassie3dBatchEnv(a.envs, device=local, control_mode=col.control_mode, auto_reset=True, max_path_length=1000)
     env.reset()
@@ -167,12 +192,20 @@ def compare_3d():
                 br[k].copy_(r); bd[k].copy_(d)
             state["obs"] = o
 
-        col.collect(sp, T); unfused(); env_only(); torch.cuda.synchronize()      # warm-up of every shape
+        dp = DeterministicMLPPolicy(col.obs_dim, col.act_dim, device=dev, hidden_sizes=shape) if ou else None
+        col.collect(sp, T); unfused(); env_only()      # warm-up of every shape
+        if ou:
+            col.collect(dp, T, es)
+        torch.cuda.synchronize()
         runs = {"fused_collect": [], "unfused_loop": [], "env_step_only": []}
+        if ou:
+            runs["fused_ou_collect"] = []
         for _ in range(2):
             runs["fused_collect"].append(timed(lambda: col.collect(sp, T), a.reps))
             runs["unfused_loop"].append(timed(unfused, a.reps))
             runs["env_step_only"].append(timed(env_only, a.reps))
+            if ou:
+                runs["fused_ou_collect"].append(timed(lambda: col.collect(dp, T, es), a.reps))
         if res is None:
             res = kernel_resources([lambda: col.collect(sp, 2), lambda: env.step(pre[0])], ["k_tree_rollout_step", "k_tree_env_step"])
         best = {k: min(v) for k, v in runs.items()}
@@ -180,15 +213,19 @@ def compare_3d():
             "ms_per_collect": runs, "env_steps_per_s": {k: [n * T * 10 / (x * 1e-3) for x in v] for k, v in runs.items()},
             "fused_vs_env_step_only": best["fused_collect"] / best["env_step_only"] - 1.0,
             "fused_vs_unfused": best["fused_collect"] / best["unfused_loop"] - 1.0}
+        if ou:
+            sweep["x".join(map(str, shape))]["ou_vs_gaussian_collect"] = best["fused_ou_collect"] / best["fused_collect"] - 1.0
     env.terminate()
     return {"hidden_sizes_sweep": sweep, "kernels": res, "card": card()}
 
 
-ms_collect = timed(lambda: col.collect(pol, a.T), a.reps)
+ms_collect = timed(lambda: col.collect(pol, a.T, es), a.reps)
 cmp3d = compare_3d() if a.model == "3d" else None
+col.collect(pol, a.T, es)                  # the buffers of the headline policy for the sampler side
+torch.cuda.synchronize()
 t0 = time.perf_counter()
 for _ in range(a.reps):
-    ret = col.discounted_returns(); col.fit_baseline(ret); col.advantages()
+    sampler_side()
 torch.cuda.synchronize()
 ms_post = maxr((time.perf_counter() - t0) / a.reps * 1e3)
 
@@ -234,12 +271,14 @@ if a.model == "3d":
     st = col.batch.stats().double()   # [n, 4]: constraint rows, contacts, PGS sweeps, contacts dropped
     if rank == 0:
         print(json.dumps({
-            "workload": "rollout: GaussianMLPPolicy(45->%s->10) + %s action space + cassie3d stand env, %d envs per GPU x %d GPUs x %d policy steps x 10 sim steps"
-                        % ("->".join(map(str, hidden)), col.control_mode, a.envs, world, a.T),
+            "workload": "rollout: %s(45->%s->10) + %s action space + cassie3d stand env, %d envs per GPU x %d GPUs x %d policy steps x 10 sim steps"
+                        % ("DeterministicMLPPolicy + OUStrategy" if ou else "GaussianMLPPolicy", "->".join(map(str, hidden)),
+                           col.control_mode, a.envs, world, a.T),
             "n_gpus": world, "collect_ms": ms_collect, "env_steps_per_s": n_total * a.T * 10 / (ms_collect * 1e-3),
             "policy_steps_per_s": n_total * a.T / (ms_collect * 1e-3),
             "env_steps_per_s_with_overlapped_gather": (n_total * a.T * 10 / (gather["collect_with_overlapped_gather_ms"] * 1e-3)) if world > 1 else None,
-            "returns_baseline_advantages_ms": ms_post, "episodes_finished": int((d != 0).sum().item()),
+            ("transitions_pool_add_random_batch256_ms" if ou else "returns_baseline_advantages_ms"): ms_post,
+            "episodes_finished": int((d != 0).sum().item()),
             "rollout_stats_all_ranks": red, "gather": gather, "compare_rank0": cmp3d,
             "last_step_rows_mean": float(st[:, 0].mean().item()), "last_step_rows_max": int(st[:, 0].max().item())}), flush=True)
     if world > 1:
